@@ -2,6 +2,8 @@
 """bench.py -- k-mers counted per second (whole job) at k=21 on synthetic 1 kb reads.
 
     python bench.py --gpus 1 --steps K --warmup W            # this repository's CUDA path
+    python bench.py ... --dump-outputs DIR                    # + the last timed step's (k-mer, count) table as .npy files
+                                                              # (seeded inputs: two builds compare output for output)
     python bench.py --impl reference --steps K --warmup W     # the reference's C functions on the host cores: every step a
                                                               # bounded sample of the same workload, sized from a calibration
                                                               # pass (--ref-seconds), + one larger pass reported beside it
@@ -118,6 +120,28 @@ def keys_unique(torch, keys):
         return all(keys_unique(torch, keys[low == r]) for r in range(pieces))
     s, _ = torch.sort(keys)
     return not bool((s[1:] == s[:-1]).any().item())
+
+
+def dump_count_table(torch, out_dir, pairs, n_kmers, suffix="", sample=1 << 20, chunk=1 << 26):
+    """--dump-outputs: the (k-mer, count) table one count call returned, as float64 .npy files two builds can be compared by.
+    The table comes back in hash order with up to one group per window (16 GB at 1 GB of random reads), so what is written is
+    the groups whose mix64(code) falls under a threshold sized for about `sample` groups -- the same groups whatever the
+    order -- sorted by code, plus the size and checksum of the whole table.  A code has 2k bits: it is stored as its high and
+    low 32-bit halves, which float64 holds exactly; so is the 64-bit checksum."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    keys, counts = pairs[:, 0], pairs[:, 1]
+    n = keys.numel()
+    thr = min(1 << 24, -(-(sample << 24) // max(n, 1)))          # compared with the top 24 bits of mix64(code)
+    picked = [pairs[i:i + chunk][((mix64_torch(torch, keys[i:i + chunk]) >> 40) & 0xffffff) < thr] for i in range(0, n, chunk)]
+    picked = torch.cat(picked) if picked else pairs[:0]
+    picked = picked[torch.argsort(picked[:, 0])][:2 * sample].cpu().numpy()
+    codes = picked[:, 0].astype(np.uint64)
+    tot, cnt = table_checksum(torch, keys, counts)
+    np.save(out / f"table_sample_codes{suffix}.npy", np.stack([codes >> np.uint64(32), codes & np.uint64(0xffffffff)], 1).astype(np.float64))
+    np.save(out / f"table_sample_counts{suffix}.npy", picked[:, 1].astype(np.float64))
+    # distinct k-mers, k-mers counted, sum of the counts, checksum (high, low 32 bits) -- see table_checksum
+    np.save(out / f"table_stats{suffix}.npy", np.array([n, n_kmers, cnt, tot >> 32, tot & 0xffffffff], dtype=np.float64))
 
 
 def input_checksum(flat, off, k):
@@ -388,6 +412,9 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the short extract / match measurements")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle checksum of the result tables (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the (k-mer, count) table of the last timed step to DIR as .npy files (a seeded sample of the "
+                         "groups plus the whole table's size and checksum, see dump_count_table)")
     ap.add_argument("--devgen", action="store_true", help="generate the reads in HBM (kmer_cuda_dev_synth_reads: one seeded table, every rank "
                                                           "its own row range) instead of on the host with numpy")
     ap.add_argument("--k", type=int, default=21, help="k-mer length of the count workload (default: the headline's 21)")
@@ -395,6 +422,10 @@ def main():
                     help="c2 = BASELINE configs[1] (default; weak scaling, --reads per GPU); c3 = configs[2]: k=31 over 10 GB in total, "
                          "strong-scaled over the GPUs; c2x10 = the north star's shape: k=21 over 10 GB in total")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "count"):
+        ap.error("--dump-outputs writes the table of the count workload of --impl b200")
     global K, METRIC
     if args.config == "c3":
         args.k = 31
@@ -513,6 +544,9 @@ def main():
         n_distinct_total = n_distinct
     ms_step = ms_total / args.steps
     value = total_kmers * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs:                              # every rank holds its own share of the groups when world > 1
+        dump_count_table(torch, args.dump_outputs, d_pairs[:int(res.n_distinct)], int(res.n_kmers),
+                         suffix=f"_rank{rank}" if world > 1 else "", sample=(1 << 20) // world)
 
     # ---------------------------------------------------------------- parity of the table the LAST timed step left in HBM
     parity = {"what": "sum(count*mix64(code)) over the table == sum(mix64(code)) over all windows of the input rows (C oracle), "

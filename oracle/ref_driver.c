@@ -228,6 +228,10 @@ Datum hash_any(const unsigned char *k, int keylen)
 	return (Datum) c;
 }
 
+/* Compiled with -DPGSHIM_NO_REFERENCE this file is the pgshim's runtime alone (palloc, ereport, SRF helpers): what a driver
+ * of the GPU glue needs when it makes no call into the reference, e.g. the planner hook's rewrite checks. */
+#ifndef PGSHIM_NO_REFERENCE
+
 /* ------------------------------------------------------------------ reference entry points */
 
 extern Datum dna_in(PG_FUNCTION_ARGS);
@@ -745,3 +749,5 @@ int ref_generate_rows(const char *flat, const uint64_t *off, uint64_t n_rows, in
 	*checksum = cs;
 	return rc;
 }
+
+#endif /* PGSHIM_NO_REFERENCE */

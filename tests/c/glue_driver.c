@@ -4,13 +4,13 @@
  * oracle/_ref/libkmer_ref.so, which also provides the shim's palloc / ereport runtime) run in the same process on the same
  * datums; the glue's datums must equal theirs BYTE FOR BYTE (header byte included, kmer.c:341-343), its counts must equal
  * the number of times the reference emitted each k-mer, its booleans the reference's booleans, its errors the reference's
- * SQLSTATE and text.  Built and run by tests/test_glue_exec.py.  Exit code 0 = all equal. */
+ * SQLSTATE and text.  Built with -DPGSHIM_NO_REFERENCE (no oracle/_ref) the expected side is the C oracle instead
+ * (tests/c/expected_kmers.h).  Built and run by tests/test_glue_exec.py.  Exit code 0 = all equal. */
 #include "postgres.h"
 #include "fmgr.h"
 #include "funcapi.h"
 #include "utils/array.h"
 
-extern Datum generate_kmers(PG_FUNCTION_ARGS);
 extern Datum kmer_equals(PG_FUNCTION_ARGS);
 extern Datum kmer_starts_with_op(PG_FUNCTION_ARGS);
 extern Datum kmer_contains(PG_FUNCTION_ARGS);
@@ -45,8 +45,7 @@ static struct varlena *make_varlena(const char *bytes, int len, int short_header
 	return v;
 }
 
-typedef struct Item { unsigned char bytes[40]; int64_t count; } Item; /* a kmer datum: header byte + <= 32 bases */
-static int cmp_item(const void *a, const void *b) { return memcmp(((const Item *) a)->bytes, ((const Item *) b)->bytes, 40); }
+#include "expected_kmers.h"
 
 static int check_counts(int n_rows, int max_len, int k, int repeat_every)
 {
@@ -62,29 +61,10 @@ static int check_counts(int n_rows, int max_len, int k, int repeat_every)
 		if (repeat_every && r % repeat_every == 0) rng_state = 42; /* the same read again: counts above 1 */
 		for (int i = 0; i < len; i++) buf[i] = "ACGTacgt"[rnd() & 7];
 		arr->elems[r] = PointerGetDatum(make_varlena(buf, len, r & 1));
-		/* the reference: one generate_kmers SRF scan of this row */
-		FunctionCallInfoBaseData fc;
-		memset(&fc, 0, sizeof(fc));
-		fc.nargs = 2;
-		/* dna_in lower-cases (kmer.c:28-29): hand the reference the stored form */
+		/* the expected side: one generate_kmers scan of this row; dna_in lower-cases (kmer.c:28-29): hand it the stored form */
 		char *low = (char *) palloc((Size) len);
 		for (int i = 0; i < len; i++) low[i] = (char) (buf[i] | 0x20);
-		fc.args[0].value = PointerGetDatum(make_varlena(low, len, 0));
-		fc.args[1].value = (Datum) k;
-		for (;;)
-		{
-			Datum d = generate_kmers(&fc);
-			if (fc.srf_done) break;
-			if (n_want == cap_want)
-			{
-				cap_want = cap_want ? cap_want * 2 : 4096;
-				want = (Item *) realloc(want, cap_want * sizeof(Item));
-			}
-			memset(&want[n_want], 0, sizeof(Item));
-			memcpy(want[n_want].bytes, DatumGetPointer(d), (size_t) k + 1); /* the datum exactly as palloc'ed */
-			want[n_want].count = 1;
-			n_want++;
-		}
+		want = expected_kmers(want, &n_want, &cap_want, low, len, k);
 	}
 	qsort(want, n_want, sizeof(Item), cmp_item);
 	size_t g = 0;
@@ -118,8 +98,8 @@ static int check_counts(int n_rows, int max_len, int k, int repeat_every)
 	qsort(got, n_got < g + 16 ? n_got : g + 16, sizeof(Item), cmp_item);
 	int ok = n_got == g;
 	for (size_t i = 0; ok && i < g; i++) ok = !memcmp(got[i].bytes, want[i].bytes, 40) && got[i].count == want[i].count;
-	printf("[glue] kmer_gpu_counts: %d rows (both header forms), k=%d: %s  groups %zu/%zu, k-mers %zu\n", n_rows, k, ok ? "ok" : "MISMATCH", n_got,
-		   g, n_want);
+	printf("[glue] kmer_gpu_counts: %d rows (both header forms), k=%d: %s  groups %zu/%zu, k-mers %zu (expected side: %s)\n", n_rows, k,
+		   ok ? "ok" : "MISMATCH", n_got, g, n_want, EXPECTED_SOURCE);
 	free(want); free(got);
 	return ok;
 }
@@ -129,14 +109,15 @@ static int check_match(int n, int op, const char *constant)
 	ArrayType *arr = (ArrayType *) palloc(sizeof(ArrayType) + (size_t) n * sizeof(Datum));
 	int ok = 1, hits = 0;
 	FunctionCallInfoBaseData fc;
-	Datum cst;
 	arr->nelems = n;
 	arr->elemtype = 0;
+#ifndef PGSHIM_NO_REFERENCE
 	/* the constant through the reference's own input function */
 	memset(&fc, 0, sizeof(fc));
 	fc.nargs = 1;
 	fc.args[0].value = PointerGetDatum(pstrdup(constant));
-	cst = op == 2 ? qkmer_in(&fc) : kmer_in(&fc);
+	Datum cst = op == 2 ? qkmer_in(&fc) : kmer_in(&fc);
+#endif
 	unsigned char *want = (unsigned char *) palloc((Size) n);
 	int clen = (int) strlen(constant);
 	for (int i = 0; i < n; i++)
@@ -149,11 +130,15 @@ static int check_match(int n, int op, const char *constant)
 				if (strchr("acgtACGT", constant[j])) b[j] = (char) (constant[j] | 0x20);
 		struct varlena *v = make_varlena(b, len, 1); /* kmer datums carry the short header (kmer.c:124-125) */
 		arr->elems[i] = PointerGetDatum(v);
+#ifdef PGSHIM_NO_REFERENCE
+		want[i] = (unsigned char) expected_match(op, b, len, constant);
+#else
 		memset(&fc, 0, sizeof(fc));
 		fc.nargs = 2;
 		if (op == 0) { fc.args[0].value = PointerGetDatum(v); fc.args[1].value = cst; want[i] = kmer_equals(&fc) != 0; }
 		else if (op == 1) { fc.args[0].value = PointerGetDatum(v); fc.args[1].value = cst; want[i] = kmer_starts_with_op(&fc) != 0; }
 		else { fc.args[0].value = cst; fc.args[1].value = PointerGetDatum(v); want[i] = kmer_contains(&fc) != 0; }
+#endif
 		hits += want[i];
 	}
 	memset(&fc, 0, sizeof(fc));
@@ -175,7 +160,7 @@ static int check_match(int n, int op, const char *constant)
 	if (first_bad >= 0)
 	{
 		struct varlena *v = (struct varlena *) DatumGetPointer(arr->elems[first_bad]);
-		printf("       first mismatch at element %d: kmer '%.*s' (len %d), reference says %d\n", first_bad, (int) VARSIZE_ANY_EXHDR(v), VARDATA_ANY(v),
+		printf("       first mismatch at element %d: kmer '%.*s' (len %d), " EXPECTED_SOURCE " says %d\n", first_bad, (int) VARSIZE_ANY_EXHDR(v), VARDATA_ANY(v),
 			   (int) VARSIZE_ANY_EXHDR(v), (int) want[first_bad]);
 	}
 	return ok;

@@ -10,7 +10,8 @@
  *   --exec (GPU)        : the REWRITTEN tree is executed by a tiny stand-in executor over a fake `reads` table -- the ARRAY
  *                         sublink scanned, kmer_gpu_counts (kmer_gpu.c) driven through the fmgr shim -- and its rows must equal,
  *                         datum for datum and count for count, what the ORIGINAL query computes with the reference's own
- *                         generate_kmers (oracle/_ref) under a sort + group.
+ *                         generate_kmers (oracle/_ref) under a sort + group -- built with -DPGSHIM_NO_REFERENCE, with the
+ *                         C oracle's generate_kmers instead (tests/c/expected_kmers.h).
  * Built and run by tests/test_hook.py.  Exit code 0 = all as expected. */
 #include "postgres.h"
 #include "fmgr.h"
@@ -22,7 +23,6 @@
 #include "utils/array.h"
 
 extern void _PG_init(void);
-extern Datum generate_kmers(PG_FUNCTION_ARGS);
 extern Datum kmer_gpu_counts(PG_FUNCTION_ARGS);
 extern void pgshim_catalog_reset(void);
 extern void pgshim_catalog_add_type(const char *name, Oid oid, Oid array_oid);
@@ -65,6 +65,8 @@ static struct varlena *make_varlena(const char *bytes, int len, int short_header
 	}
 	return v;
 }
+
+#include "expected_kmers.h"
 
 static Const *int4_const(int v)
 {
@@ -398,9 +400,6 @@ static void structure_tests(void)
 }
 
 /* ------------------------------------------------------------------ the rewritten tree executed (GPU) */
-typedef struct Item { unsigned char bytes[40]; int64_t count; } Item;
-static int cmp_item(const void *a, const void *b) { return memcmp(((const Item *) a)->bytes, ((const Item *) b)->bytes, 40); }
-
 static uint64_t rng_state = 0x2545F4914F6CDD1DULL;
 static uint32_t rnd(void)
 {
@@ -416,7 +415,7 @@ static int row_qualifies(Node *quals, int id)
 	return ((OpExpr *) quals)->opno == OP_ID_IS_EVEN ? id % 2 == 0 : 0;
 }
 
-/* what the ORIGINAL query computes: generate_kmers over every qualifying row (the reference, oracle/_ref), sort, group */
+/* what the ORIGINAL query computes: generate_kmers over every qualifying row (the reference, or the C oracle), sort, group */
 static size_t reference_groups(const FakeTable *t, Node *quals, struct varlena *const_dna, int k, Item **out)
 {
 	Item *want = NULL;
@@ -429,21 +428,7 @@ static size_t reference_groups(const FakeTable *t, Node *quals, struct varlena *
 		int len = VARSIZE_ANY_EXHDR(src);
 		char *low = (char *) palloc((Size) len + 1);
 		for (int i = 0; i < len; i++) low[i] = (char) (VARDATA_ANY(src)[i] | 0x20); /* dna_in lower-cases, kmer.c:28-29 */
-		FunctionCallInfoBaseData fc;
-		memset(&fc, 0, sizeof(fc));
-		fc.nargs = 2;
-		fc.args[0].value = PointerGetDatum(make_varlena(low, len, 0));
-		fc.args[1].value = (Datum) k;
-		for (;;)
-		{
-			Datum d = generate_kmers(&fc);
-			if (fc.srf_done) break;
-			if (n == cap) { cap = cap ? cap * 2 : 4096; want = (Item *) realloc(want, cap * sizeof(Item)); }
-			memset(&want[n], 0, sizeof(Item));
-			memcpy(want[n].bytes, DatumGetPointer(d), (size_t) k + 1);
-			want[n].count = 1;
-			n++;
-		}
+		want = expected_kmers(want, &n, &cap, low, len, k);
 	}
 	qsort(want, n, sizeof(Item), cmp_item);
 	for (size_t i = 0; i < n; i++)
@@ -522,7 +507,7 @@ static void exec_case(const char *what, Query *q, const FakeTable *t, Node *orig
 	int ok = n == g;
 	for (size_t i = 0; ok && i < g; i++) ok = !memcmp(got[i].bytes, want[i].bytes, 40) && got[i].count == want[i].count;
 	char line[200];
-	snprintf(line, sizeof(line), "%s: rewritten plan on the GPU == original query via the reference (%zu/%zu groups)", what, n, g);
+	snprintf(line, sizeof(line), "%s: rewritten plan on the GPU == original query via " EXPECTED_SOURCE " (%zu/%zu groups)", what, n, g);
 	CHECK(ok, line);
 	free(want); free(got);
 }

@@ -45,3 +45,14 @@ def count_canon_from_codes(keys: np.ndarray, counts: np.ndarray, k: int) -> byte
 
 def generate_canon_from_codes(codes: np.ndarray, k: int) -> bytes:
     return O.np_decode(codes, k).tobytes()
+
+
+def expected_side_link_args() -> list:
+    """gcc arguments for the expected side of tests/c/{glue,hook}_driver.c (tests/c/expected_kmers.h): the reference's own
+    functions where oracle/_ref is built, else the C oracle (pinned to the reference's answers by test_oracle.py) with the
+    pgshim runtime of oracle/ref_driver.c"""
+    O.build(ref=True)
+    if O.REF_SO.exists():
+        return [f"-L{O.REF_SO.parent}", "-lkmer_ref", f"-Wl,-rpath,{O.REF_SO.parent}"]
+    return ["-DPGSHIM_NO_REFERENCE", "-Wno-unused-function", str(O.HERE / "ref_driver.c"), f"-L{O.HERE}", "-lkmer_oracle",
+            f"-Wl,-rpath,{O.HERE}"]

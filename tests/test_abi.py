@@ -141,6 +141,62 @@ def test_bench_reference_arm_prints_one_json_line():
     assert out.returncode == 0 and not [ln for ln in out.stdout.splitlines() if ln.startswith("{")]
 
 
+def test_bench_dump_outputs_do_not_depend_on_table_order(tmp_path):
+    """bench.py --dump-outputs: the same table in any order gives the same files, all float64; the sampled codes (64-bit at
+    k=32), their counts and the whole table's checksum come back exactly"""
+    import importlib.util
+    import numpy as np
+    import torch
+    from oracle import oracle as O
+    spec = importlib.util.spec_from_file_location("bench_module", ROOT / "bench.py")
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    rng = np.random.default_rng(3)
+    keys = np.unique(rng.integers(-(1 << 63), (1 << 63) - 1, 300_000, dtype=np.int64))
+    counts = rng.integers(1, 9, keys.size, dtype=np.int64)
+    pairs = torch.from_numpy(np.stack([keys, counts], 1))
+    outs = []
+    for i, p in enumerate((pairs, pairs[torch.randperm(keys.size, generator=torch.Generator().manual_seed(1))])):
+        bench.dump_count_table(torch, tmp_path / str(i), p, int(counts.sum()), sample=1 << 12)
+        outs.append({f.name: np.load(f) for f in (tmp_path / str(i)).iterdir()})
+    assert outs[0].keys() == {"table_sample_codes.npy", "table_sample_counts.npy", "table_stats.npy"}
+    for name, a in outs[0].items():
+        assert a.dtype == np.float64 and np.array_equal(a, outs[1][name]), name
+    hi_lo = outs[0]["table_sample_codes.npy"].astype(np.uint64)
+    codes = ((hi_lo[:, 0] << np.uint64(32)) | hi_lo[:, 1]).view(np.int64)
+    assert 3000 < codes.size < 6000 and np.all(codes[1:] > codes[:-1])
+    at = np.searchsorted(keys, codes)
+    assert np.array_equal(keys[at], codes) and np.array_equal(outs[0]["table_sample_counts.npy"], counts[at])
+    n, n_kmers, cnt, hi, lo = (int(x) for x in outs[0]["table_stats.npy"])
+    assert n == keys.size and n_kmers == cnt == int(counts.sum())
+    assert (hi << 32 | lo) == O.np_table_checksum(keys.view(np.uint64), counts.astype(np.uint64))
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_hold_the_counted_table(tmp_path):
+    """`bench.py --dump-outputs` on the GPU: the files appear, their statistics are those of the table the JSON line reports,
+    and the sample -- the whole table while it has at most 2^20 groups -- is the oracle's GROUP BY of the same seeded reads"""
+    import json, subprocess, sys
+    import numpy as np
+    from kmer_extension_b200 import datagen
+    from oracle import oracle as O
+    reads = 1000                                   # 980 000 windows: under the 2^20 groups of the sample
+    cmd = [sys.executable, str(ROOT / "bench.py"), "--gpus", "1", "--reads", str(reads), "--steps", "2", "--warmup", "3",
+           "--no-e2e", "--no-cpu", "--no-secondary", "--dump-outputs", str(tmp_path)]
+    out = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = json.loads([ln for ln in out.stdout.splitlines() if ln.startswith("{")][-1])
+    assert d["steps"] == 2 and d["parity"]["checksum_ok"] and d["parity"]["count_ok"]
+    flat, off = datagen.synth_reads(2, reads, 1000)
+    keys, counts, n = O.np_count(flat, off, 21)
+    s, _ = O.COracle().multiset_checksum(flat, off, 21)
+    stats = [int(x) for x in np.load(tmp_path / "table_stats.npy")]
+    assert stats == [keys.size, n, n, s >> 32, s & 0xffffffff] and d["config"]["n_distinct_rank0"] == keys.size
+    hi_lo = np.load(tmp_path / "table_sample_codes.npy").astype(np.uint64)
+    assert np.array_equal((hi_lo[:, 0] << np.uint64(32)) | hi_lo[:, 1], keys)
+    assert np.array_equal(np.load(tmp_path / "table_sample_counts.npy"), counts.astype(np.float64))
+
+
 def test_pg_regress_suite_is_generated_from_the_kats():
     """kmer-extension_b200/pgglue/regress/{sql,expected} are what tools/make_pg_regress.py derives from tests/golden/kat.json"""
     import subprocess, sys
