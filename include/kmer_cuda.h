@@ -140,6 +140,17 @@ int kmer_cuda_submit_count_packed(kmer_cuda_ctx *ctx, const char *seq, const uin
 								  uint8_t **uniq_packed, uint64_t *n_unique, int *code_bytes, kmer_count_pair **pairs,
 								  uint64_t *n_pairs, uint64_t *n_kmers);
 
+/* The k-mer abundance spectrum (count of counts) of the same GROUP BY -- what `jellyfish histo`, KAT and GenomeScope work from:
+ *   SELECT cnt AS count, count(*) AS kmers
+ *   FROM (SELECT count(*) AS cnt FROM reads r, generate_kmers(r.dna, k) AS g(kmer) GROUP BY g.kmer) s GROUP BY cnt
+ * (*hist)[c], 1 <= c < hist_len (>= 2): number of distinct k-mers counted exactly c times; (*hist)[0] = 0.  Every group whose
+ * count is >= hist_len comes back whole in (*tail)[0..*n_tail), in unspecified order (the high-copy k-mers themselves), so
+ * the spectrum is exact for any count.  The groups are binned on the device: no buffer of the table's size exists on either
+ * side of PCIe.  Same errors as kmer_cuda_submit_count.  Both results are released with kmer_cuda_release(). */
+int kmer_cuda_submit_count_spectrum(kmer_cuda_ctx *ctx, const char *seq, const uint64_t *row_off, uint64_t n_rows, int k,
+									uint64_t hist_len, uint64_t **hist, kmer_count_pair **tail, uint64_t *n_tail,
+									uint64_t *n_kmers);
+
 /* Replaces per-row calls of kmer_equals / kmer_starts_with[_op] / kmer_contains / kmer_containing
  * (kmer.c:226-285) over a column of m k-mers against n_consts constants given as text:
  *   KMER_OP_EQUALS, KMER_OP_STARTS_WITH : constants are kmer literals   (kmer_in rules, kmer.c:109-129)
@@ -198,6 +209,18 @@ int kmer_cuda_dev_count(kmer_cuda_ctx *ctx, const char *d_seq, uint64_t n_bases,
 int kmer_cuda_dev_count_split(kmer_cuda_ctx *ctx, const char *d_seq, uint64_t n_bases, const uint64_t *d_row_off,
 							  uint64_t n_rows, int k, uint64_t *d_uniq, uint64_t uniq_capacity, kmer_count_pair *d_pairs,
 							  uint64_t pairs_capacity, void *stream);
+
+/* Spectrum result format (see kmer_cuda_submit_count_spectrum): d_hist[0..hist_len) is overwritten whole (hist_len >= 2), the
+ * groups with count >= hist_len are written to d_tail; floor(n_windows / hist_len) entries always suffice, fewer than needed fail
+ * with KMER_ERR_CAPACITY.  kmer_cuda_dev_finish() reports n_kmers = windows counted, n_distinct = tail entries written,
+ * n_tier2 / n_overflow as for kmer_cuda_dev_count, n_unique = 0.  algo as kmer_cuda_dev_count (1 = dense, 2 = hash, 3 / 4 =
+ * partition; 0 = dense for k <= 13, partition for k >= 14); same errors. */
+int kmer_cuda_dev_count_spectrum(kmer_cuda_ctx *ctx, const char *d_seq, uint64_t n_bases, const uint64_t *d_row_off,
+								 uint64_t n_rows, int k, uint64_t *d_hist, uint64_t hist_len, kmer_count_pair *d_tail,
+								 uint64_t tail_capacity, int algo, void *stream);
+/* The spectrum of a (k-mer, count) table already in HBM, d_pairs[0..n): same outputs and finish() report. */
+int kmer_cuda_dev_pairs_spectrum(kmer_cuda_ctx *ctx, const kmer_count_pair *d_pairs, uint64_t n, uint64_t *d_hist,
+								 uint64_t hist_len, kmer_count_pair *d_tail, uint64_t tail_capacity, void *stream);
 
 /* consts / ops are HOST arrays (they are compiled to masks on the host); d_* are device pointers.
  * d_bits: n_consts * ceil(m/32) words; d_hits: n_consts counters. */
@@ -277,6 +300,13 @@ int kmer_cuda_dev_shard_count_split(kmer_cuda_ctx *ctx, const kmer_shard_plan *p
 int kmer_cuda_dev_shard_count_peers(kmer_cuda_ctx *ctx, const kmer_shard_plan *plan, const void *const *src_recs,
 									const uint64_t *const *src_fill, uint64_t *d_uniq, uint64_t uniq_capacity,
 									kmer_count_pair *d_pairs, uint64_t pairs_capacity, void *stream);
+/* This rank's share of sharded counting in the spectrum result format (kmer_cuda_dev_count_spectrum), sources given as in
+ * kmer_cuda_dev_shard_count_peers.  After the all-to-all, the receive buffers are passed in the same form:
+ * src_recs[s] = (char *)recv_recs + s * plan->recs_bytes_per_peer, src_fill[s] = recv_fill + s * plan->buckets_per_rank.
+ * The owners' groups are disjoint: the ranks' histograms sum, and their tails concatenate, to the spectrum of all rows. */
+int kmer_cuda_dev_shard_count_spectrum(kmer_cuda_ctx *ctx, const kmer_shard_plan *plan, const void *const *src_recs,
+									   const uint64_t *const *src_fill, uint64_t *d_hist, uint64_t hist_len,
+									   kmer_count_pair *d_tail, uint64_t tail_capacity, void *stream);
 /* CUDA IPC for one-process-per-GPU hosts: export names the cudaMalloc ALLOCATION d_ptr lies in (handle64: 64 bytes to
  * send to the peers) and d_ptr's offset inside it; open maps a peer's allocation into this process (enabling peer
  * access from ctx's GPU) and returns its base; close unmaps it.  A handle can be open once per process. */

@@ -44,6 +44,7 @@ ABI_SYMBOLS = [
     "kmer_cuda_dev_merge_begin", "kmer_cuda_dev_merge_add", "kmer_cuda_dev_merge_emit", "kmer_cuda_test_force_window",
     "kmer_cuda_init_multi", "kmer_cuda_shutdown_multi", "kmer_cuda_multi_device_count", "kmer_cuda_multi_last_error",
     "kmer_cuda_multi_submit_count", "kmer_cuda_multi_release", "kmer_cuda_dev_pack_codes", "kmer_cuda_multi_submit_match", "kmer_cuda_dev_synth_reads",
+    "kmer_cuda_dev_count_spectrum", "kmer_cuda_dev_shard_count_spectrum", "kmer_cuda_dev_pairs_spectrum", "kmer_cuda_submit_count_spectrum",
 ]
 
 
@@ -125,6 +126,10 @@ def load_library(path: Path = LIB_PATH) -> C.CDLL:
     L.kmer_cuda_dev_merge_add.argtypes = [vp, vp, u64, C.c_uint32, C.c_uint32, vp]
     L.kmer_cuda_dev_merge_emit.argtypes = [vp, i32, vp, u64, vp]
     L.kmer_cuda_dev_synth_reads.argtypes = [vp, u64, u64, u64, u64, vp, vp, vp]
+    L.kmer_cuda_dev_count_spectrum.argtypes = [vp, vp, u64, vp, u64, i32, vp, u64, vp, u64, i32, vp]
+    L.kmer_cuda_dev_shard_count_spectrum.argtypes = [vp, C.POINTER(KmerShardPlan), C.POINTER(vp), C.POINTER(vp), vp, u64, vp, u64, vp]
+    L.kmer_cuda_dev_pairs_spectrum.argtypes = [vp, vp, u64, vp, u64, vp, u64, vp]
+    L.kmer_cuda_submit_count_spectrum.argtypes = [vp, vp, vp, u64, i32, u64, C.POINTER(vp), C.POINTER(vp), u64p, u64p]
     return L
 
 
@@ -139,6 +144,19 @@ def _flat(rows_or_flat, off=None):
     if bs:
         o[1:] = np.cumsum([len(b) for b in bs], dtype=np.uint64)
     return np.frombuffer(b"".join(bs), dtype=np.uint8), o
+
+
+def spectrum_rows(hist, tail):
+    """The SQL relation of the abundance spectrum -- `SELECT cnt AS count, count(*) AS kmers FROM (... GROUP BY kmer) s GROUP BY
+    cnt ORDER BY cnt` -- from a histogram (hist[c] = k-mers counted c times, c < len(hist)) and the tail of groups whose count is
+    >= len(hist) (an [n, 2] (code, count) array, or just their counts): (count, kmers) uint64 arrays, ascending by count, zero
+    rows omitted."""
+    hist = np.asarray(hist, dtype=np.uint64).reshape(-1)
+    tail = np.asarray(tail, dtype=np.uint64)
+    tcounts = tail[:, 1] if tail.ndim == 2 else tail.reshape(-1)
+    c = np.nonzero(hist)[0].astype(np.uint64)
+    tc, tk = np.unique(tcounts, return_counts=True)
+    return np.concatenate([c, tc.astype(np.uint64)]), np.concatenate([hist[c.astype(np.int64)], tk.astype(np.uint64)])
 
 
 class KmerCuda:
@@ -244,6 +262,17 @@ class KmerCuda:
         a = self._take(pairs, npairs.value * 16, np.uint64).reshape(-1, 2)
         return u, a[:, 0].copy(), a[:, 1].copy(), int(n.value), int(nb.value)
 
+    def count_spectrum(self, rows_or_flat, k: int, off=None, hist_len: int = 65536):
+        """Abundance spectrum of the GROUP BY -> (hist[hist_len] uint64, tail [n, 2] uint64 (code, count) of the groups with
+        count >= hist_len, order unspecified); spectrum_rows(hist, tail) is the SQL relation."""
+        f, o = _flat(rows_or_flat, off)
+        hist, tail, nt, n = C.c_void_p(), C.c_void_p(), C.c_uint64(), C.c_uint64()
+        self._check(self.lib.kmer_cuda_submit_count_spectrum(self.ctx, f.ctypes.data, o.ctypes.data, len(o) - 1, k, hist_len,
+                                                             C.byref(hist), C.byref(tail), C.byref(nt), C.byref(n)))
+        h = self._take(hist, hist_len * 8, np.uint64)
+        t = self._take(tail, nt.value * 16, np.uint64).reshape(-1, 2)
+        return h, t
+
     def match(self, op, codes: np.ndarray, k: int, consts, lens: np.ndarray | None = None, ops=None):
         """Bit matrix [n_consts, m] (bool) and hits[n_consts] for the column `codes`."""
         codes = np.ascontiguousarray(codes, dtype=np.uint64)
@@ -326,6 +355,18 @@ class KmerCuda:
                                                        d_uniq.data_ptr(), d_uniq.numel(), d_pairs.data_ptr(), d_pairs.numel() // 2,
                                                        self._stream_ptr(stream)))
 
+    def dev_count_spectrum(self, d_seq, n_bases: int, d_off, n_rows: int, k: int, d_hist, d_tail, algo: int = ALGO_AUTO, stream=None):
+        """Spectrum result format: d_hist uint64/int64 [hist_len] (overwritten whole), d_tail [tail_capacity, 2] gets the groups
+        with count >= hist_len; dev_finish().n_distinct = tail entries written."""
+        self._check(self.lib.kmer_cuda_dev_count_spectrum(self.ctx, d_seq.data_ptr(), n_bases, d_off.data_ptr(), n_rows, k,
+                                                          d_hist.data_ptr(), d_hist.numel(), d_tail.data_ptr(), d_tail.shape[0], algo,
+                                                          self._stream_ptr(stream)))
+
+    def dev_pairs_spectrum(self, d_pairs, n: int, d_hist, d_tail, stream=None):
+        """The spectrum of the (code, count) table d_pairs[:n] (same outputs as dev_count_spectrum)."""
+        self._check(self.lib.kmer_cuda_dev_pairs_spectrum(self.ctx, d_pairs.data_ptr(), n, d_hist.data_ptr(), d_hist.numel(),
+                                                          d_tail.data_ptr(), d_tail.shape[0], self._stream_ptr(stream)))
+
     def dev_match(self, op, d_codes, m: int, k: int, consts, d_bits, d_hits, d_lens=None, ops=None, stream=None):
         consts = [consts] if isinstance(consts, str) else list(consts)
         arr = (C.c_char_p * max(len(consts), 1))(*[s.encode() for s in consts])
@@ -376,6 +417,15 @@ class KmerCuda:
         self._check(self.lib.kmer_cuda_dev_shard_count_peers(
             self.ctx, C.byref(plan), a_r, a_f, d_uniq.data_ptr() if d_uniq is not None else None,
             d_uniq.numel() if d_uniq is not None else 0, d_pairs.data_ptr(), d_pairs.numel() // 2, self._stream_ptr(stream)))
+
+    def dev_shard_count_spectrum(self, plan: KmerShardPlan, src_recs, src_fill, d_hist, d_tail, stream=None):
+        """This rank's share in the spectrum format; src_recs / src_fill: device ADDRESSES (ints) of every source's segments for
+        this rank -- the peers' send blocks, or recv_recs + s * recs_bytes_per_peer / recv_fill + s * buckets_per_rank * 8."""
+        n = len(src_recs)
+        a_r = (C.c_void_p * n)(*[int(x) for x in src_recs])
+        a_f = (C.c_void_p * n)(*[int(x) for x in src_fill])
+        self._check(self.lib.kmer_cuda_dev_shard_count_spectrum(self.ctx, C.byref(plan), a_r, a_f, d_hist.data_ptr(), d_hist.numel(),
+                                                                d_tail.data_ptr(), d_tail.shape[0], self._stream_ptr(stream)))
 
     def ipc_export(self, d_tensor):
         """(64-byte handle of the allocation the tensor lies in, the tensor's byte offset inside it)"""

@@ -27,7 +27,8 @@ struct PinnedBuf {
     bool in_use;
 };
 
-enum PendingOp { OP_NONE = 0, OP_EXTRACT, OP_COUNT, OP_MATCH, OP_DECODE, OP_ENCODE, OP_SHARD_PART, OP_SHARD_COUNT, OP_DENSE_TABLE, OP_MERGE };
+enum PendingOp { OP_NONE = 0, OP_EXTRACT, OP_COUNT, OP_MATCH, OP_DECODE, OP_ENCODE, OP_SHARD_PART, OP_SHARD_COUNT, OP_DENSE_TABLE, OP_MERGE,
+                 OP_PAIRS_SPECTRUM };
 
 }  // namespace
 
@@ -43,7 +44,7 @@ struct kmer_cuda_ctx {
     cudaEvent_t ev_in[8] = {}, ev_leaf[16] = {}, ev_off = nullptr;
     DevStatus* h_ring = nullptr;    // pinned: status snapshots behind every group of buckets
     // device workspaces, grown on demand and kept between calls
-    Buf seq, off, mask, tile_row, table, consts, ops, codes, pairs, bits, hits, lens, text, fill, recs, spill, failed, seg, segfill;
+    Buf seq, off, mask, tile_row, table, consts, ops, codes, pairs, bits, hits, lens, text, fill, recs, spill, failed, seg, segfill, hist;
     uint64_t merge_slots = 0;     // table slots of the merge in progress (kmer_cuda_dev_merge_*)
     uint64_t last_tier2 = 0;      // k-mers counted by the tier-2 kernel in the last count
     uint64_t last_overflow = 0;   // k-mers the partition counter could not place (batch was recounted)
@@ -60,6 +61,12 @@ struct kmer_cuda_ctx {
     const uint64_t* p_off = nullptr;
     kmer_count_pair* p_pairs = nullptr;
     uint64_t p_pairs_cap = 0;
+    // ... or, in the spectrum result format, re-zeroes the histogram and rebins into it (the tail cursor is DevStatus::n_distinct)
+    bool p_spectrum = false;
+    uint64_t* p_hist = nullptr;
+    uint64_t p_hist_len = 0;
+    kmer_count_pair* p_tail = nullptr;
+    uint64_t p_tail_cap = 0;
     // optional phase timing (bench.py's per-kernel roofline): events recorded after each phase
     bool profiling = false;
     std::vector<cudaEvent_t> ev_pool;
@@ -367,7 +374,7 @@ extern "C" void kmer_cuda_shutdown(kmer_cuda_ctx* c) {
     cudaSetDevice(c->di.device);
     if (c->stream) cudaStreamSynchronize(c->stream);
     Buf* all[] = {&c->seq, &c->off, &c->mask, &c->tile_row, &c->table, &c->consts, &c->ops,
-                  &c->codes, &c->pairs, &c->bits, &c->hits, &c->lens, &c->text, &c->fill, &c->recs, &c->spill, &c->failed, &c->seg, &c->segfill};
+                  &c->codes, &c->pairs, &c->bits, &c->hits, &c->lens, &c->text, &c->fill, &c->recs, &c->spill, &c->failed, &c->seg, &c->segfill, &c->hist};
     for (Buf* b : all) buf_free(*b);
     for (auto& p : c->pinned) cudaFreeHost(p.p);
     for (auto e : c->ev_pool) cudaEventDestroy(e);
@@ -435,6 +442,7 @@ static int begin_op(kmer_cuda_ctx* c, cudaStream_t st, bool keep_input_findings 
     c->launches++;
     c->pending = OP_NONE;
     c->p_recountable = false;
+    c->p_spectrum = false;
     return KMER_OK;
 }
 
@@ -505,10 +513,21 @@ static uint64_t next_pow2(uint64_t v) {
     return p;
 }
 
-// d_uniq != nullptr: split result format (see kmer_cuda_dev_count_split)
+static SpecOut spec_out(uint64_t* d_hist, uint64_t hist_len, kmer_count_pair* d_tail, uint64_t tail_capacity) {
+    return SpecOut{reinterpret_cast<unsigned long long*>(d_hist), hist_len, d_tail, tail_capacity};
+}
+
+// the spectrum result format: the histogram is overwritten whole (the tail cursor is reset by begin_op)
+static int spectrum_begin(kmer_cuda_ctx* c, const SpecOut& o, cudaStream_t st) {
+    CU(cudaMemsetAsync(o.hist, 0, o.hist_len * sizeof(uint64_t), st), "memset hist");
+    return KMER_OK;
+}
+
+// d_uniq != nullptr: split result format (see kmer_cuda_dev_count_split); spec != nullptr: spectrum result format
+// (kmer_cuda_dev_count_spectrum; d_pairs / d_uniq unused)
 static int dev_count_impl(kmer_cuda_ctx* c, const char* d_seq, uint64_t n_bases, const uint64_t* d_row_off, uint64_t n_rows, int k,
                           kmer_count_pair* d_pairs, uint64_t pairs_capacity, uint64_t* d_uniq, uint64_t uniq_capacity, int algo,
-                          void* stream) {
+                          void* stream, const SpecOut* spec = nullptr) {
     if (!c) return KMER_ERR_BAD_ARGUMENT;
     cudaStream_t st = pick_stream(c, stream);
     int rc = begin_op(c, st);
@@ -516,6 +535,10 @@ static int dev_count_impl(kmer_cuda_ctx* c, const char* d_seq, uint64_t n_bases,
     c->pending = OP_COUNT;
     c->p_n_bases = n_bases; c->p_n_rows = n_rows; c->p_k = k;
     c->p_expected_kmers = kmer_cuda_max_kmers(n_bases, n_rows, k);
+    if (spec) {
+        rc = spectrum_begin(c, *spec, st);
+        if (rc) return rc;
+    }
     if (n_rows == 0 || n_bases == 0) {
         if (n_rows) return ref_error(&c->err, KMER_ERR_INVALID_K, 0);
         return KMER_OK;
@@ -548,21 +571,26 @@ static int dev_count_impl(kmer_cuda_ctx* c, const char* d_seq, uint64_t n_bases,
             launch_scatter_refine(c->di, a, plan, sp, (uint32_t*)c->segfill.p, c->seg.p, (unsigned long long*)c->fill.p, c->recs.p,
                                   c->spill.p, st, mark_cb, &ma);
             launch_bucket_count(c->di, plan, k, (const unsigned long long*)c->fill.p, c->recs.p, c->spill.p, (uint32_t*)c->failed.p, d_pairs,
-                                pairs_capacity, d_uniq, uniq_capacity, c->d_status, st);
+                                pairs_capacity, d_uniq, uniq_capacity, c->d_status, st, 0, 0, spec);
             mark(c, st, "bucket_count");
             c->launches += 3;
         } else {
             launch_count_partition(c->di, a, plan, (unsigned long long*)c->fill.p, c->recs.p, c->spill.p, (uint32_t*)c->failed.p,
-                                   d_pairs, pairs_capacity, d_uniq, uniq_capacity, st, mark_cb, &ma);
+                                   d_pairs, pairs_capacity, d_uniq, uniq_capacity, st, mark_cb, &ma, spec);
             c->launches += 2;
         }
         // Tier 2 (buckets that did not fit on chip, spilled records) is decided and run by the device: nothing here waits
         // for the GPU.  Only a batch that overflows even that (DevStatus::n_overflow) is recounted, by kmer_cuda_dev_finish.
         launch_partition_tier2(c->di, plan, k, (const unsigned long long*)c->fill.p, c->recs.p, c->spill.p, (const uint32_t*)c->failed.p,
-                               (kmer_count_pair*)c->table.p, t2_slots, d_pairs, pairs_capacity, c->d_status, st, mark_cb, &ma);
+                               (kmer_count_pair*)c->table.p, t2_slots, d_pairs, pairs_capacity, c->d_status, st, mark_cb, &ma, spec);
         c->launches += 4;
         c->p_recountable = true;
         c->p_seq = d_seq; c->p_off = d_row_off; c->p_pairs = d_pairs; c->p_pairs_cap = pairs_capacity;
+        c->p_spectrum = spec != nullptr;
+        if (spec) {
+            c->p_hist = reinterpret_cast<uint64_t*>(spec->hist); c->p_hist_len = spec->hist_len;
+            c->p_tail = spec->tail; c->p_tail_cap = spec->tail_cap;
+        }
         algo = -1;
     }
     if (algo == 1) {
@@ -570,9 +598,13 @@ static int dev_count_impl(kmer_cuda_ctx* c, const char* d_seq, uint64_t n_bases,
         uint64_t nbins = 1ull << (2 * k);
         rc = ws(c, c->table, nbins * 8);
         if (rc) return rc;
-        launch_count_dense(c->di, a, (unsigned long long*)c->table.p, d_pairs, pairs_capacity, st);
+        if (spec) {
+            launch_dense_table(c->di, a, (unsigned long long*)c->table.p, st);
+            launch_dense_spectrum(c->di, (const unsigned long long*)c->table.p, k, 0, 1, *spec, c->d_status, st);
+        } else
+            launch_count_dense(c->di, a, (unsigned long long*)c->table.p, d_pairs, pairs_capacity, st);
         c->launches += 2;
-        mark(c, st, "count_dense+compact");
+        mark(c, st, spec ? "count_dense+spectrum" : "count_dense+compact");
     } else if (algo == 2) {
         uint64_t maxd = c->p_expected_kmers;
         if (k < 32 && (1ull << (2 * k)) < maxd) maxd = 1ull << (2 * k);
@@ -583,9 +615,10 @@ static int dev_count_impl(kmer_cuda_ctx* c, const char* d_seq, uint64_t n_bases,
         mark(c, st, "hash_clear");
         launch_count_hash_insert(c->di, a, (kmer_count_pair*)c->table.p, n_slots, st);
         mark(c, st, "count_hash_insert");
-        launch_hash_compact(c->di, (const kmer_count_pair*)c->table.p, n_slots, k, d_pairs, pairs_capacity, c->d_status, st);
+        if (spec) launch_hash_spectrum(c->di, (const kmer_count_pair*)c->table.p, n_slots, k, *spec, c->d_status, st);
+        else launch_hash_compact(c->di, (const kmer_count_pair*)c->table.p, n_slots, k, d_pairs, pairs_capacity, c->d_status, st);
         c->launches += 2;
-        mark(c, st, "hash_compact");
+        mark(c, st, spec ? "hash_spectrum" : "hash_compact");
     } else if (algo != -1)
         return bad_arg(c, "unknown counting algorithm");
     resolve_bad_row_kernel<<<1, 1, 0, st>>>(c->d_status, d_row_off, n_rows);
@@ -606,6 +639,44 @@ extern "C" int kmer_cuda_dev_count_split(kmer_cuda_ctx* c, const char* d_seq, ui
     if (c && !d_uniq && uniq_capacity) return bad_arg(c, "d_uniq");
     return dev_count_impl(c, d_seq, n_bases, d_row_off, n_rows, k, d_pairs, pairs_capacity, d_uniq, d_uniq ? uniq_capacity : 0, 0,
                           stream);
+}
+
+static int spectrum_args(kmer_cuda_ctx* c, const uint64_t* d_hist, uint64_t hist_len, const kmer_count_pair* d_tail, uint64_t tail_capacity) {
+    if (!d_hist || hist_len < 2) return bad_arg(c, "d_hist / hist_len (>= 2)");
+    if (!d_tail && tail_capacity) return bad_arg(c, "d_tail");
+    return KMER_OK;
+}
+
+extern "C" int kmer_cuda_dev_count_spectrum(kmer_cuda_ctx* c, const char* d_seq, uint64_t n_bases, const uint64_t* d_row_off,
+                                            uint64_t n_rows, int k, uint64_t* d_hist, uint64_t hist_len, kmer_count_pair* d_tail,
+                                            uint64_t tail_capacity, int algo, void* stream) {
+    if (!c) return KMER_ERR_BAD_ARGUMENT;
+    int rc = spectrum_args(c, d_hist, hist_len, d_tail, tail_capacity);
+    if (rc) return rc;
+    const SpecOut o = spec_out(d_hist, hist_len, d_tail, tail_capacity);
+    return dev_count_impl(c, d_seq, n_bases, d_row_off, n_rows, k, nullptr, 0, nullptr, 0, algo, stream, &o);
+}
+
+extern "C" int kmer_cuda_dev_pairs_spectrum(kmer_cuda_ctx* c, const kmer_count_pair* d_pairs, uint64_t n, uint64_t* d_hist,
+                                            uint64_t hist_len, kmer_count_pair* d_tail, uint64_t tail_capacity, void* stream) {
+    if (!c) return KMER_ERR_BAD_ARGUMENT;
+    int rc = spectrum_args(c, d_hist, hist_len, d_tail, tail_capacity);
+    if (rc) return rc;
+    if (n && !d_pairs) return bad_arg(c, "d_pairs");
+    cudaStream_t st = pick_stream(c, stream);
+    rc = begin_op(c, st);
+    if (rc) return rc;
+    c->pending = OP_PAIRS_SPECTRUM;
+    const SpecOut o = spec_out(d_hist, hist_len, d_tail, tail_capacity);
+    rc = spectrum_begin(c, o, st);
+    if (rc) return rc;
+    if (n) {
+        launch_pairs_spectrum(c->di, d_pairs, n, o, c->d_status, st);
+        c->launches++;
+        mark(c, st, "pairs_spectrum");
+    }
+    CU(cudaGetLastError(), "pairs spectrum launch");
+    return KMER_OK;
 }
 
 static int upload_consts(kmer_cuda_ctx* c, int op, const int* ops, const char* const* consts, uint32_t n_consts,
@@ -748,10 +819,16 @@ extern "C" int kmer_cuda_dev_finish(kmer_cuda_ctx* c, void* stream, kmer_dev_res
             a.row_mask = (const uint32_t*)c->mask.p;
             a.k = k;
             a.status = c->d_status;
-            status_reset_kernel<<<1, 1, 0, st>>>(c->d_status);
+            status_reset_kernel<<<1, 1, 0, st>>>(c->d_status);          // also rewinds the tail cursor of the spectrum format
             launch_hash_clear((kmer_count_pair*)c->table.p, n_slots, st);
             launch_count_hash_insert(c->di, a, (kmer_count_pair*)c->table.p, n_slots, st);
-            launch_hash_compact(c->di, (const kmer_count_pair*)c->table.p, n_slots, k, c->p_pairs, c->p_pairs_cap, c->d_status, st);
+            if (c->p_spectrum) {                                        // what the leaf and tier 2 binned so far is void as well
+                const SpecOut o = spec_out(c->p_hist, c->p_hist_len, c->p_tail, c->p_tail_cap);
+                rc = spectrum_begin(c, o, st);
+                if (rc) return rc;
+                launch_hash_spectrum(c->di, (const kmer_count_pair*)c->table.p, n_slots, k, o, c->d_status, st);
+            } else
+                launch_hash_compact(c->di, (const kmer_count_pair*)c->table.p, n_slots, k, c->p_pairs, c->p_pairs_cap, c->d_status, st);
             c->launches += 3;
             CU(cudaMemcpyAsync(c->h_status, c->d_status, sizeof(DevStatus), cudaMemcpyDeviceToHost, st), "D2H status");
             CU(cudaStreamSynchronize(st), "stream sync");
@@ -800,7 +877,7 @@ extern "C" int kmer_cuda_dev_finish(kmer_cuda_ctx* c, void* stream, kmer_dev_res
             result->n_tier2 = c->last_tier2;
             result->n_unique = s.n_unique;
         }
-    } else if (op == OP_MERGE) {
+    } else if (op == OP_MERGE || op == OP_PAIRS_SPECTRUM) {
         if (s.out_overflow)
             return set_error(&c->err, KMER_ERR_CAPACITY, "XX000", "kmer_cuda: output buffer too small", "", -1);
         if (s.n_overflow)
@@ -910,7 +987,8 @@ extern "C" int kmer_cuda_dev_shard_partition(kmer_cuda_ctx* c, const char* d_seq
 }
 
 static int dev_shard_count_impl(kmer_cuda_ctx* c, const kmer_shard_plan* sp, const SrcTable& src, uint64_t* d_uniq,
-                                uint64_t uniq_capacity, kmer_count_pair* d_pairs, uint64_t pairs_capacity, void* stream) {
+                                uint64_t uniq_capacity, kmer_count_pair* d_pairs, uint64_t pairs_capacity, void* stream,
+                                const SpecOut* spec = nullptr) {
     cudaStream_t st = pick_stream(c, stream);
     const bool chained = c->pending == OP_SHARD_PART;    // no finish since the partition: its findings stay in the status block
     int rc = begin_op(c, st, chained);
@@ -923,6 +1001,10 @@ static int dev_shard_count_impl(kmer_cuda_ctx* c, const kmer_shard_plan* sp, con
     if ((sp->cap & 1u) || sp->fine_shift > 12) return bad_arg(c, "shard plan: cap must be even, fine_shift <= 12");
     // coarse partitions (one segment per source GPU) -> this GPU's fine buckets, then counted like a single-GPU batch
     PartitionPlan plan = fine_partition_plan(sp);
+    if (spec) {
+        rc = spectrum_begin(c, *spec, st);
+        if (rc) return rc;
+    }
     rc = ws(c, c->fill, (size_t)plan.n_buckets * 8);
     if (!rc) rc = ws(c, c->recs, partition_record_bytes(plan));
     if (!rc) rc = ws(c, c->spill, partition_spill_bytes(plan));
@@ -933,7 +1015,7 @@ static int dev_shard_count_impl(kmer_cuda_ctx* c, const kmer_shard_plan* sp, con
                   c->d_status, st);
     mark(c, st, "refine");
     launch_bucket_count(c->di, plan, k, (const unsigned long long*)c->fill.p, c->recs.p, c->spill.p, (uint32_t*)c->failed.p, d_pairs,
-                        pairs_capacity, d_uniq, d_uniq ? uniq_capacity : 0, c->d_status, st);
+                        pairs_capacity, d_uniq, d_uniq ? uniq_capacity : 0, c->d_status, st, 0, 0, spec);
     mark(c, st, "bucket_count");
     c->launches += 2;
     // tier 2 is decided and run by the device (no host round trip); an overflow of even that is reported by finish()
@@ -942,7 +1024,7 @@ static int dev_shard_count_impl(kmer_cuda_ctx* c, const kmer_shard_plan* sp, con
     if (rc) return rc;
     MarkArg ma{c, st};
     launch_partition_tier2(c->di, plan, k, (const unsigned long long*)c->fill.p, c->recs.p, c->spill.p, (const uint32_t*)c->failed.p,
-                           (kmer_count_pair*)c->table.p, t2_slots, d_pairs, pairs_capacity, c->d_status, st, mark_cb, &ma);
+                           (kmer_count_pair*)c->table.p, t2_slots, d_pairs, pairs_capacity, c->d_status, st, mark_cb, &ma, spec);
     c->launches += 4;
     CU(cudaGetLastError(), "shard count launch");
     return KMER_OK;
@@ -995,6 +1077,28 @@ extern "C" int kmer_cuda_dev_shard_count_peers(kmer_cuda_ctx* c, const kmer_shar
         src.fill[s] = (const unsigned long long*)src_fill[s];
     }
     return dev_shard_count_impl(c, sp, src, d_uniq, uniq_capacity, d_pairs, pairs_capacity, stream);
+}
+
+// This rank's share in the spectrum result format.  The owners' groups are disjoint, so the ranks' histograms add up and their
+// tails concatenate to the spectrum of the whole job.  The exchanged layout is the same form: src_recs[s] = recv_recs + s *
+// recs_bytes_per_peer, src_fill[s] = recv_fill + s * buckets_per_rank.
+extern "C" int kmer_cuda_dev_shard_count_spectrum(kmer_cuda_ctx* c, const kmer_shard_plan* sp, const void* const* src_recs,
+                                                  const uint64_t* const* src_fill, uint64_t* d_hist, uint64_t hist_len,
+                                                  kmer_count_pair* d_tail, uint64_t tail_capacity, void* stream) {
+    if (!c || !sp) return KMER_ERR_BAD_ARGUMENT;
+    int rc = spectrum_args(c, d_hist, hist_len, d_tail, tail_capacity);
+    if (rc) return rc;
+    if (!src_recs || !src_fill) return bad_arg(c, "src_recs / src_fill");
+    const uint32_t n_src = sp->n_ranks * (sp->chunks_per_rank ? sp->chunks_per_rank : 1u);
+    if (n_src > (uint32_t)KMER_MAX_SRC) return bad_arg(c, "shard plan: too many sources");
+    SrcTable src{};
+    for (uint32_t s = 0; s < n_src; s++) {
+        if (!src_recs[s] || !src_fill[s]) return bad_arg(c, "src_recs / src_fill: null entry");
+        src.recs[s] = src_recs[s];
+        src.fill[s] = (const unsigned long long*)src_fill[s];
+    }
+    const SpecOut o = spec_out(d_hist, hist_len, d_tail, tail_capacity);
+    return dev_shard_count_impl(c, sp, src, nullptr, 0, nullptr, 0, stream, &o);
 }
 
 // ---- CUDA IPC: a device buffer of this process opened in another process on the same node (one process per GPU)
@@ -1179,15 +1283,16 @@ extern "C" int kmer_cuda_submit_extract(kmer_cuda_ctx* c, const char* seq, const
     return KMER_OK;
 }
 
-// ---- GROUP BY through host buffers: one implementation for the three result formats ------------------------------------------
-enum CountFormat { FMT_PAIRS = 0, FMT_SPLIT = 1, FMT_PACKED = 2 };
+// ---- GROUP BY through host buffers: one implementation for the four result formats -------------------------------------------
+enum CountFormat { FMT_PAIRS = 0, FMT_SPLIT = 1, FMT_PACKED = 2, FMT_SPECTRUM = 3 };
 
-struct CountOut {              // what the three entry points hand back
+struct CountOut {              // what the four entry points hand back
     void* uniq = nullptr;      // SPLIT: uint64 codes; PACKED: code_bytes-byte integers
     uint64_t n_unique = 0;
     int code_bytes = 0;
-    kmer_count_pair* pairs = nullptr;
+    kmer_count_pair* pairs = nullptr;   // SPECTRUM: the tail
     uint64_t n_pairs = 0, n_kmers = 0;
+    uint64_t* hist = nullptr;           // SPECTRUM: hist_len counters
 };
 
 // a pinned result buffer that goes back to the pool unless it is handed to the caller (no leak on any error return)
@@ -1240,12 +1345,30 @@ static int download_count_result(kmer_cuda_ctx* c, int k, CountFormat fmt, const
     return KMER_OK;
 }
 
+// The spectrum format: the histogram and the tail -> pinned host memory.
+static int download_spectrum(kmer_cuda_ctx* c, uint64_t hist_len, const kmer_dev_result& res, CountOut* o) {
+    PinGuard gh(c), gt(c);
+    gh.p = pinned_get(c, hist_len * sizeof(uint64_t));
+    if (!gh.p) return c->err.status;
+    CU(cudaMemcpyAsync(gh.p, c->hist.p, hist_len * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream), "D2H hist");
+    gt.p = pinned_get(c, res.n_distinct * sizeof(kmer_count_pair));
+    if (!gt.p) return c->err.status;
+    CU(cudaMemcpyAsync(gt.p, c->pairs.p, res.n_distinct * sizeof(kmer_count_pair), cudaMemcpyDeviceToHost, c->stream), "D2H tail");
+    CU(cudaStreamSynchronize(c->stream), "stream sync");
+    o->hist = (uint64_t*)gh.take();
+    o->pairs = (kmer_count_pair*)gt.take();
+    o->n_pairs = res.n_distinct;
+    o->n_kmers = res.n_kmers;
+    return KMER_OK;
+}
+
 // Replaces the scan + HashAggregate of a whole column (kmer.c:289-351 + kmer_hash/kmer_equals) from HOST buffers.  For
 // 14 <= k <= 32 the three legs overlap: the column arrives in pieces on a copy stream while the pieces already there are
 // partitioned; the buckets are counted in groups, and behind every group the part of the result that is final leaves on a
-// second copy stream (PCIe is the bound of this call: the kernels hide under the copies).
+// second copy stream (PCIe is the bound of this call: the kernels hide under the copies).  FMT_SPECTRUM (hist_len >= 2): the
+// groups are binned on the device and nothing streams back but the histogram and the tail, once everything is counted.
 static int submit_count_common(kmer_cuda_ctx* c, const char* seq, const uint64_t* row_off, uint64_t n_rows, int k, CountFormat fmt,
-                               CountOut* o) {
+                               CountOut* o, uint64_t hist_len = 0) {
     CU(cudaSetDevice(c->di.device), "cudaSetDevice");
     if (n_rows && !row_off) return bad_arg(c, "row_off");
     const uint64_t n_bases = n_rows ? row_off[n_rows] : 0;
@@ -1257,17 +1380,29 @@ static int submit_count_common(kmer_cuda_ctx* c, const char* seq, const uint64_t
     uint64_t cap = kmer_cuda_max_kmers(n_bases, n_rows, k);
     if (k >= 1 && k < 32 && (1ull << (2 * k)) < cap) cap = 1ull << (2 * k);
     // a k-mer that is not unique occurs at least twice: at most cap/2 pairs next to the unique codes -- unless a fallback
-    // tier (which writes pairs only) takes over, so the pair buffer keeps the full size
-    rc = ws(c, c->pairs, cap * sizeof(kmer_count_pair));
-    if (!rc && fmt != FMT_PAIRS) rc = ws(c, c->codes, cap * sizeof(uint64_t));
+    // tier (which writes pairs only) takes over, so the pair buffer keeps the full size.  The spectrum format needs no buffer
+    // of the table's size: at most n_windows / hist_len groups reach the tail.
+    const bool spectrum = fmt == FMT_SPECTRUM;
+    const uint64_t tail_cap = spectrum ? std::max<uint64_t>(1, kmer_cuda_max_kmers(n_bases, n_rows, k) / hist_len) : 0;
+    if (spectrum) {
+        rc = ws(c, c->pairs, tail_cap * sizeof(kmer_count_pair));
+        if (!rc) rc = ws(c, c->hist, hist_len * sizeof(uint64_t));
+    } else {
+        rc = ws(c, c->pairs, cap * sizeof(kmer_count_pair));
+        if (!rc && fmt != FMT_PAIRS) rc = ws(c, c->codes, cap * sizeof(uint64_t));
+    }
     if (rc) return rc;
+    const SpecOut so = spec_out((uint64_t*)c->hist.p, hist_len, (kmer_count_pair*)c->pairs.p, tail_cap);
     const bool pipelined = k >= 14 && k <= KMER_CUDA_MAX_K && n_rows && n_bases >= (4ull << 20);
     kmer_dev_result res;
     if (!pipelined) {
         rc = h2d(c, c->seq.p, seq, n_bases, c->stream);
         if (!rc && n_rows) rc = h2d(c, c->off.p, row_off, (n_rows + 1) * 8, c->stream);
         if (rc) return rc;
-        if (fmt == FMT_PAIRS)
+        if (spectrum)
+            rc = kmer_cuda_dev_count_spectrum(c, (const char*)c->seq.p, n_bases, (const uint64_t*)c->off.p, n_rows, k, (uint64_t*)c->hist.p,
+                                              hist_len, (kmer_count_pair*)c->pairs.p, tail_cap, 0, KMER_OWN_STREAM);
+        else if (fmt == FMT_PAIRS)
             rc = kmer_cuda_dev_count(c, (const char*)c->seq.p, n_bases, (const uint64_t*)c->off.p, n_rows, k, (kmer_count_pair*)c->pairs.p, cap,
                                      0, KMER_OWN_STREAM);
         else
@@ -1276,7 +1411,7 @@ static int submit_count_common(kmer_cuda_ctx* c, const char* seq, const uint64_t
         if (rc) return rc;
         rc = kmer_cuda_dev_finish(c, KMER_OWN_STREAM, &res);
         if (rc) return rc;
-        return download_count_result(c, k, fmt, res, o);
+        return spectrum ? download_spectrum(c, hist_len, res, o) : download_count_result(c, k, fmt, res, o);
     }
 
     // ---------------------------------------------------------------- pipelined: copy-in | kernels | copy-out
@@ -1286,7 +1421,7 @@ static int submit_count_common(kmer_cuda_ctx* c, const char* seq, const uint64_t
     const char* d_seq = (const char*)c->seq.p;
     const uint64_t* d_off = (const uint64_t*)c->off.p;
     kmer_count_pair* d_pairs = (kmer_count_pair*)c->pairs.p;
-    uint64_t* d_uniq = fmt == FMT_PAIRS ? nullptr : (uint64_t*)c->codes.p;
+    uint64_t* d_uniq = fmt == FMT_PAIRS || spectrum ? nullptr : (uint64_t*)c->codes.p;
     const int nbytes = (2 * k + 7) / 8;
     const size_t ubytes = fmt == FMT_PACKED ? (size_t)nbytes : 8;
     if (fmt == FMT_PACKED) {
@@ -1295,8 +1430,10 @@ static int submit_count_common(kmer_cuda_ctx* c, const char* seq, const uint64_t
     }
     // the result buffer the final ranges stream into: sized for the most the batch can produce
     PinGuard gout(c);
-    gout.p = pinned_get(c, fmt == FMT_PAIRS ? cap * sizeof(kmer_count_pair) : cap * ubytes);
-    if (!gout.p) return c->err.status;
+    if (!spectrum) {
+        gout.p = pinned_get(c, fmt == FMT_PAIRS ? cap * sizeof(kmer_count_pair) : cap * ubytes);
+        if (!gout.p) return c->err.status;
+    }
     // 1. offsets first: the row mask needs nothing else
     CU(cudaMemcpyAsync(c->off.p, row_off, (n_rows + 1) * 8, cudaMemcpyHostToDevice, c->s_in), "H2D offsets");
     CU(cudaEventRecord(c->ev_off, c->s_in), "event");
@@ -1308,6 +1445,10 @@ static int submit_count_common(kmer_cuda_ctx* c, const char* seq, const uint64_t
     c->p_expected_kmers = kmer_cuda_max_kmers(n_bases, n_rows, k);
     c->last_overflow = 0;
     c->last_tier2 = 0;
+    if (spectrum) {
+        rc = spectrum_begin(c, so, st);
+        if (rc) return rc;
+    }
     ScanArgs a;
     rc = prepare_rows(c, d_off, n_bases, n_rows, k, st, &a, d_seq);
     if (rc) return rc;
@@ -1336,25 +1477,35 @@ static int submit_count_common(kmer_cuda_ctx* c, const char* seq, const uint64_t
         c->launches++;
     }
     mark(c, st, "minimizer_partition");
-    // 3. the buckets in groups; behind every group a snapshot of the result cursors
-    const int n_groups = plan.n_buckets >= 4096 ? 8 : 1;
+    // 3. the buckets in groups; behind every group a snapshot of the result cursors (the spectrum format: one launch, nothing
+    //    streams back before the end)
+    const SpecOut* spec = spectrum ? &so : nullptr;
+    const int n_groups = !spectrum && plan.n_buckets >= 4096 ? 8 : 1;
     for (int g = 0; g < n_groups; g++) {
         const uint32_t g0 = (uint32_t)((uint64_t)plan.n_buckets * g / n_groups), g1 = (uint32_t)((uint64_t)plan.n_buckets * (g + 1) / n_groups);
         launch_bucket_count(c->di, plan, k, (const unsigned long long*)c->fill.p, c->recs.p, c->spill.p, (uint32_t*)c->failed.p, d_pairs,
-                            cap, d_uniq, d_uniq ? cap : 0, c->d_status, st, g0, g1);
+                            cap, d_uniq, d_uniq ? cap : 0, c->d_status, st, g0, g1, spec);
         c->launches++;
+        if (spectrum) break;
         CU(cudaMemcpyAsync(&c->h_ring[g], c->d_status, sizeof(DevStatus), cudaMemcpyDeviceToHost, st), "D2H status");
         CU(cudaEventRecord(c->ev_leaf[g], st), "event");
     }
     mark(c, st, "bucket_count");
     MarkArg ma{c, st};
     launch_partition_tier2(c->di, plan, k, (const unsigned long long*)c->fill.p, c->recs.p, c->spill.p, (const uint32_t*)c->failed.p,
-                           (kmer_count_pair*)c->table.p, t2_slots, d_pairs, cap, c->d_status, st, mark_cb, &ma);
+                           (kmer_count_pair*)c->table.p, t2_slots, d_pairs, cap, c->d_status, st, mark_cb, &ma, spec);
     resolve_bad_row_kernel<<<1, 1, 0, st>>>(c->d_status, d_off, n_rows);
     c->launches += 5;
     CU(cudaGetLastError(), "count launch");
     c->p_recountable = true;
     c->p_seq = d_seq; c->p_off = d_off; c->p_pairs = d_pairs; c->p_pairs_cap = cap;
+    c->p_spectrum = spectrum;
+    if (spectrum) {
+        c->p_hist = (uint64_t*)c->hist.p; c->p_hist_len = hist_len; c->p_tail = d_pairs; c->p_tail_cap = tail_cap;
+        rc = kmer_cuda_dev_finish(c, KMER_OWN_STREAM, &res);      // input errors, tier 2, or a tier-3 recount
+        if (rc) return rc;
+        return download_spectrum(c, hist_len, res, o);
+    }
     // 4. while later groups are counted, what the finished ones wrote leaves (everything below a snapshot's cursor is final)
     uint64_t done = 0;                                             // entries of the streamed array already on their way
     bool input_error = false;
@@ -1462,6 +1613,23 @@ extern "C" int kmer_cuda_submit_count_packed(kmer_cuda_ctx* c, const char* seq, 
     *code_bytes = k >= 1 ? (2 * k + 7) / 8 : 1;
     *pairs = o.pairs;
     *n_pairs = o.n_pairs;
+    if (n_kmers) *n_kmers = o.n_kmers;
+    return KMER_OK;
+}
+
+extern "C" int kmer_cuda_submit_count_spectrum(kmer_cuda_ctx* c, const char* seq, const uint64_t* row_off, uint64_t n_rows, int k,
+                                             uint64_t hist_len, uint64_t** hist, kmer_count_pair** tail, uint64_t* n_tail,
+                                             uint64_t* n_kmers) {
+    if (!c || !hist || !tail || !n_tail || hist_len < 2) return KMER_ERR_BAD_ARGUMENT;
+    *hist = nullptr; *tail = nullptr;
+    *n_tail = 0;
+    if (n_kmers) *n_kmers = 0;
+    CountOut o;
+    int rc = submit_count_common(c, seq, row_off, n_rows, k, FMT_SPECTRUM, &o, hist_len);
+    if (rc) return rc;
+    *hist = o.hist;
+    *tail = o.pairs;
+    *n_tail = o.n_pairs;
     if (n_kmers) *n_kmers = o.n_kmers;
     return KMER_OK;
 }

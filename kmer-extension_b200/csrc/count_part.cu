@@ -28,7 +28,7 @@
 #include <cmath>
 #include <cstdlib>
 
-#include "kernels.cuh"
+#include "spectrum.cuh"
 
 namespace kmer {
 
@@ -285,6 +285,10 @@ __global__ void __launch_bounds__(NT, PART_MINB) partition_kernel(ScanArgs a, Pa
 //   emit    : unique k-mers straight from the registers, table entries from the claimed-slot lists (which also
 //             resets the table); both as coalesced 16-byte (k-mer, count) pairs (or bare codes in the split format).
 //             Output ranges: one global atomicAdd per bucket for the unique k-mers, one per warp that claimed slots.
+//   SPEC    : the spectrum result format (count of counts, spectrum.cuh) instead of the groups: the unique k-mers are only
+//             counted (a register per warp, added to the CTA's bin 1 at the end), table entries are binned in the CTA's shared
+//             histogram (counts < 64), into hist[] (counts < hist_len) or appended to the tail; no output range is handed out
+//             and nothing is stored per group.  out / capacity are the tail, out_u / capacity_u the histogram and its length.
 // Buckets above LEAF_MAX_KMERS, or whose region overflowed in the partition pass, go to tier 2 up front.
 // Shared memory is addressed through explicit 32-bit shared addresses (ld/st/atom.shared PTX).
 
@@ -392,7 +396,7 @@ __device__ __forceinline__ BucketInfo bucket_info(const unsigned long long* __re
     return bi;
 }
 
-template <int RECW, bool SPLIT>
+template <int RECW, bool SPLIT, bool SPEC = false>
 __global__ void __launch_bounds__(LEAF_THREADS, LEAF_MINB) bucket_count_kernel(PartitionPlan plan, int k,
                                                                        const unsigned long long* __restrict__ fill,
                                                                        const Rec<RECW>* __restrict__ recs,
@@ -413,6 +417,7 @@ __global__ void __launch_bounds__(LEAF_THREADS, LEAF_MINB) bucket_count_kernel(P
     const uint32_t p_s = slow_s + LEAF_KEYS * 2;                               // u16[cap + 2]: first key index of every record
     const uint32_t rec0_s = p_s + ((((uint32_t)plan.cap + 2u) * 2u + 15u) & ~15u);   // staged records, two buffers
     const uint32_t rec_stride = (((uint32_t)plan.cap + 2u) * RECB + 15u) & ~15u;
+    const uint32_t hist_s = rec0_s + 2u * rec_stride;                          // SPEC: u32[SPEC_SBINS]
     __shared__ __align__(8) uint64_t s_mbar;
     __shared__ uint32_t s_mask[2][LEAF_BLOCKS];                                // per bucket parity: bit i&31 of word i>>5: a record starts at key index i
     __shared__ uint32_t s_blk[LEAF_BLOCKS];                                    // record that covers key index 32*block
@@ -434,6 +439,9 @@ __global__ void __launch_bounds__(LEAF_THREADS, LEAF_MINB) bucket_count_kernel(P
     if (t < LEAF_BLOCKS) { s_mask[0][t] = 0; s_mask[1][t] = 0; }
     if (t < 2) { s_nuniq[t] = 0; s_nslow[t] = 0; }
     if (t == 0) { s_kcur = 0; mbar_init(&s_mbar, 1); mbar_fence_init(); }
+    if (SPEC)
+        for (int i = t; i < SPEC_SBINS; i += LEAF_THREADS) sts32(hist_s + 4 * i, 0u);
+    uint32_t uniq_total = 0;                                            // SPEC: unique k-mers of this warp (the same on every lane)
     __syncthreads();
 
     // thread 0: start the bulk copy of bucket b's records (padded to 16 bytes; read once: L2 evict-first)
@@ -562,12 +570,15 @@ __global__ void __launch_bounds__(LEAF_THREADS, LEAF_MINB) bucket_count_kernel(P
         // the warp's unique k-mers get a contiguous share of the bucket's output
         const uint32_t wuniq = __reduce_add_sync(0xffffffffu, (uint32_t)__popc(uniq));
         uint32_t woff = 0;
-        if (lane == 0 && wuniq) woff = atoms_add32(smem_u32(&s_nuniq[par]), wuniq);
-        woff = __shfl_sync(0xffffffffu, woff, 0);
+        if (SPEC) uniq_total += wuniq;
+        else {
+            if (lane == 0 && wuniq) woff = atoms_add32(smem_u32(&s_nuniq[par]), wuniq);
+            woff = __shfl_sync(0xffffffffu, woff, 0);
+        }
         __syncthreads();                                                // (L) slow list complete
         const uint32_t ns = s_nslow[par];
         unsigned long long ubase = 0;
-        if (t == 0) {
+        if (t == 0 && !SPEC) {
             const uint32_t nu = s_nuniq[par];
             if (nu) ubase = atomicAdd(SPLIT ? &status->n_unique : &status->n_distinct, (unsigned long long)nu);   // consumed after the next barrier
         }
@@ -631,14 +642,14 @@ __global__ void __launch_bounds__(LEAF_THREADS, LEAF_MINB) bucket_count_kernel(P
             }
         }
         unsigned long long wbase = 0;
-        if (lane == 0 && nwin) wbase = atomicAdd(&status->n_distinct, (unsigned long long)nwin);
+        if (lane == 0 && nwin && !SPEC) wbase = atomicAdd(&status->n_distinct, (unsigned long long)nwin);
         if (t == 0) s_obase[par] = ubase;
         if (RECW == 2) special_total += special;
         __syncthreads();                                                // (B) all counts final
         if (t < 2) { if (t == 0) s_nuniq[par ^ 1] = 0; else s_nslow[par ^ 1] = 0; }   // idle until the next bucket's classify phase
         if (t >= 32 && t < 32 + LEAF_BLOCKS) s_mask[par][t - 32] = 0;   // this bucket's start bits: idle until the bucket after the next
         // ---- emit the unique k-mers: coalesced 16-byte (k-mer, 1) pairs, ranks by ballot
-        {
+        if (!SPEC) {
             const unsigned long long ob = s_obase[par] + woff;
             const bool fits = ob + wuniq <= (SPLIT ? capacity_u : capacity);   // uniform per warp
             if (!fits && lane == 0) status->out_overflow = 1;
@@ -665,6 +676,27 @@ __global__ void __launch_bounds__(LEAF_THREADS, LEAF_MINB) bucket_count_kernel(P
             }
         }
         // ---- emit + reset the table entries this warp claimed
+        if (SPEC) {
+            const SpecOut so{reinterpret_cast<unsigned long long*>(out_u), capacity_u, out, capacity};
+            for (uint32_t i0 = 0; i0 < nwin; i0 += 32) {               // whole warps: spectrum_bin_warp is warp-collective
+                const uint32_t i = i0 + lane;
+                uint64_t code = 0, cnt = 0;
+                if (i < nwin) {
+                    const uint32_t h = lds16(slow_s + 2 * (kb + i));
+                    const unsigned long long v = lds64(tbl_s + 8 * h);
+                    sts64(tbl_s + 8 * h, kEmpty);
+                    unsigned long long c;
+                    if (PACKED) c = v >> 52;
+                    else {
+                        c = lds32(cnt_s + 4 * h);
+                        if (c) sts32(cnt_s + 4 * h, 0u);
+                    }
+                    code = v & KEYMASK;
+                    cnt = 1ull + c;
+                }
+                spectrum_bin_warp(hist_s, so, status, code, cnt);
+            }
+        } else {
         wbase = __shfl_sync(0xffffffffu, wbase, 0);
         for (uint32_t i = lane; i < nwin; i += 32) {
             const uint32_t h = lds16(slow_s + 2 * (kb + i));
@@ -680,6 +712,7 @@ __global__ void __launch_bounds__(LEAF_THREADS, LEAF_MINB) bucket_count_kernel(P
             if (idx < capacity) { ulonglong2 o; o.x = v & KEYMASK; o.y = 1ull + c; reinterpret_cast<ulonglong2*>(out)[idx] = o; }
             else status->out_overflow = 1;
         }
+        }
         if (t == 0) kmers_total += cur.nk;
         par ^= 1;
         rb ^= 1u;
@@ -694,6 +727,11 @@ __global__ void __launch_bounds__(LEAF_THREADS, LEAF_MINB) bucket_count_kernel(P
         }
     }
     if (t == 0 && kmers_total) atomicAdd(&status->n_kmers, kmers_total);
+    if (SPEC) {                                                         // the unique k-mers into bin 1, then the CTA's bins out
+        if (lane == 0 && uniq_total) reds_add32(hist_s + 4, uniq_total);
+        __syncthreads();
+        spectrum_flush(hist_s, SpecOut{reinterpret_cast<unsigned long long*>(out_u), capacity_u, out, capacity});
+    }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1217,16 +1255,17 @@ size_t leaf_smem_bytes(const PartitionPlan& p) {
     return fixed + 2 * ((staged + 15) & ~(size_t)15);                     // two record buffers
 }
 
-// once per process and device: opt in to the leaf's dynamic shared memory
+// once per process and device: opt in to the leaf's dynamic shared memory (the spectrum format adds its bins)
 static void leaf_configure(size_t smem) {
     static size_t configured[64] = {};
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev < 0 || dev >= 64 || configured[dev] >= smem) return;
-#define KMER_LEAF_CONF(RW, SP)                                                                                   \
-    cudaFuncSetAttribute(bucket_count_kernel<RW, SP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-    cudaFuncSetAttribute(bucket_count_kernel<RW, SP>, cudaFuncAttributePreferredSharedMemoryCarveout, 100)
+#define KMER_LEAF_CONF(RW, ...)                                                                                         \
+    cudaFuncSetAttribute(bucket_count_kernel<RW, __VA_ARGS__>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem + SPEC_SBINS * 4); \
+    cudaFuncSetAttribute(bucket_count_kernel<RW, __VA_ARGS__>, cudaFuncAttributePreferredSharedMemoryCarveout, 100)
     KMER_LEAF_CONF(1, false); KMER_LEAF_CONF(1, true); KMER_LEAF_CONF(2, false); KMER_LEAF_CONF(2, true);
+    KMER_LEAF_CONF(1, false, true); KMER_LEAF_CONF(2, false, true);
 #undef KMER_LEAF_CONF
     configured[dev] = smem;
 }
@@ -1234,16 +1273,26 @@ static void leaf_configure(size_t smem) {
 void launch_bucket_count(const DeviceInfo& di, const PartitionPlan& p, int k, const unsigned long long* d_fill,
                          const void* d_recs, void* d_spill, uint32_t* d_failed_ids, kmer_count_pair* d_pairs, uint64_t capacity,
                          uint64_t* d_uniq, uint64_t uniq_capacity, DevStatus* d_status, cudaStream_t st, uint32_t bucket_begin,
-                         uint32_t bucket_end) {
+                         uint32_t bucket_end, const SpecOut* spec) {
     if (bucket_end == 0 || bucket_end > p.n_buckets) bucket_end = p.n_buckets;
     if (bucket_begin >= bucket_end) return;
-    const size_t leaf_smem = leaf_smem_bytes(p);
+    const size_t leaf_smem = leaf_smem_bytes(p) + (spec ? SPEC_SBINS * 4 : 0);
     int per_sm = (int)((size_t)227 * 1024 / (leaf_smem + 1024));
     if (per_sm > LEAF_MINB) per_sm = LEAF_MINB;
     if (per_sm < 1) per_sm = 1;
     uint64_t lgrid = (uint64_t)di.sm_count * per_sm;
     if (lgrid > bucket_end - bucket_begin) lgrid = bucket_end - bucket_begin;
-    leaf_configure(leaf_smem);
+    leaf_configure(leaf_smem_bytes(p));
+    if (spec) {
+#define KMER_LEAF_SPEC(RW)                                                                                                        \
+    bucket_count_kernel<RW, false, true><<<(unsigned)lgrid, LEAF_THREADS, leaf_smem, st>>>(                                        \
+        p, k, d_fill, (const Rec<RW>*)d_recs, spec->tail, spec->tail_cap, reinterpret_cast<uint64_t*>(spec->hist), spec->hist_len, \
+        d_failed_ids, (Rec<RW>*)d_spill, d_status, bucket_begin, bucket_end)
+        if (p.recw == 1) KMER_LEAF_SPEC(1);
+        else KMER_LEAF_SPEC(2);
+#undef KMER_LEAF_SPEC
+        return;
+    }
 #define KMER_LEAF_GO(RW, SP)                                                                                                            \
     bucket_count_kernel<RW, SP><<<(unsigned)lgrid, LEAF_THREADS, leaf_smem, st>>>(p, k, d_fill, (const Rec<RW>*)d_recs, d_pairs, capacity, \
                                                                                   d_uniq, uniq_capacity, d_failed_ids, (Rec<RW>*)d_spill, d_status, bucket_begin, bucket_end)
@@ -1254,10 +1303,12 @@ void launch_bucket_count(const DeviceInfo& di, const PartitionPlan& p, int k, co
 
 void launch_count_partition(const DeviceInfo& di, const ScanArgs& a, const PartitionPlan& p, unsigned long long* d_fill,
                             void* d_recs, void* d_spill, uint32_t* d_failed_ids, kmer_count_pair* d_pairs, uint64_t capacity,
-                            uint64_t* d_uniq, uint64_t uniq_capacity, cudaStream_t st, void (*mark)(void*, const char*), void* mark_arg) {
+                            uint64_t* d_uniq, uint64_t uniq_capacity, cudaStream_t st, void (*mark)(void*, const char*), void* mark_arg,
+                            const SpecOut* spec) {
     launch_partition(di, a, p, d_fill, d_recs, d_spill, st);
     if (mark) mark(mark_arg, "minimizer_partition");
-    launch_bucket_count(di, p, a.k, d_fill, d_recs, d_spill, d_failed_ids, d_pairs, capacity, d_uniq, uniq_capacity, a.status, st);
+    launch_bucket_count(di, p, a.k, d_fill, d_recs, d_spill, d_failed_ids, d_pairs, capacity, d_uniq, uniq_capacity, a.status, st, 0, 0,
+                        spec);
     if (mark) mark(mark_arg, "bucket_count");
 }
 
@@ -1270,7 +1321,7 @@ uint64_t tier2_table_slots(uint64_t n_kmers) {
 void launch_partition_tier2(const DeviceInfo& di, const PartitionPlan& p, int k, const unsigned long long* d_fill,
                             const void* d_recs, const void* d_spill, const uint32_t* d_failed_ids, kmer_count_pair* d_slots,
                             uint64_t n_slots, kmer_count_pair* d_pairs, uint64_t capacity, DevStatus* d_status, cudaStream_t st,
-                            void (*mark)(void*, const char*), void* mark_arg) {
+                            void (*mark)(void*, const char*), void* mark_arg, const SpecOut* spec) {
     const unsigned grid = (unsigned)di.sm_count * 8;
     tier2_decide_kernel<<<1, 1, 0, st>>>(p, n_slots, d_status);
     tier2_clear_kernel<<<grid, 256, 0, st>>>((uint4*)d_slots, d_status);
@@ -1281,8 +1332,9 @@ void launch_partition_tier2(const DeviceInfo& di, const PartitionPlan& p, int k,
         tier2_insert_kernel<2><<<grid, 256, 0, st>>>(p, k, d_fill, (const Rec<2>*)d_recs, d_failed_ids, (const Rec<2>*)d_spill,
                                                      d_slots, d_status);
     if (mark) mark(mark_arg, "tier2_insert");
-    launch_hash_compact(di, d_slots, n_slots, k, d_pairs, capacity, d_status, st, 1);   // + the k == 32 special key
-    if (mark) mark(mark_arg, "tier2_compact");
+    if (spec) launch_hash_spectrum(di, d_slots, n_slots, k, *spec, d_status, st, 1);   // + the k == 32 special key
+    else launch_hash_compact(di, d_slots, n_slots, k, d_pairs, capacity, d_status, st, 1);
+    if (mark) mark(mark_arg, spec ? "tier2_spectrum" : "tier2_compact");
 }
 
 void launch_refine(const DeviceInfo& di, const PartitionPlan& p, int k, int n_src, uint32_t n_coarse, uint32_t coarse_cap,

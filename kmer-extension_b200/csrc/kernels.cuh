@@ -13,6 +13,14 @@ struct DeviceInfo {
     size_t total_mem;
 };
 
+// the abundance spectrum as a result format (spectrum.cuh): hist[0..hist_len) counters, tail[0..tail_cap) pairs
+struct SpecOut {
+    unsigned long long* hist;
+    uint64_t hist_len;
+    kmer_count_pair* tail;
+    uint64_t tail_cap;
+};
+
 // rows.cu ---------------------------------------------------------------------------------------
 // zeroes + fills the row-start mask, flags rows shorter than k (or non-monotone offsets)
 void launch_rows_prepare(const uint64_t* d_off, uint64_t n_rows, uint64_t n_bases, int k, uint32_t* d_mask,
@@ -46,6 +54,15 @@ void launch_merge_pairs(const DeviceInfo& di, const kmer_count_pair* d_in, uint6
 // appends every occupied slot (+ the k==32 special key) to d_pairs, bumping status->n_distinct
 void launch_hash_compact(const DeviceInfo& di, const kmer_count_pair* d_slots, uint64_t n_slots, int k,
                          kmer_count_pair* d_pairs, uint64_t capacity, DevStatus* d_status, cudaStream_t st, int gated = 0);
+
+// spectrum.cu: the spectrum of a table in HBM -- hash table slots (gated: tier 2's, + the k == 32 special key, as
+// launch_hash_compact), the dense 4^k counters (bins owned by `rank`), or (k-mer, count) pairs
+void launch_hash_spectrum(const DeviceInfo& di, const kmer_count_pair* d_slots, uint64_t n_slots, int k, const SpecOut& o,
+                          DevStatus* d_status, cudaStream_t st, int gated = 0);
+void launch_dense_spectrum(const DeviceInfo& di, const unsigned long long* d_table, int k, uint32_t rank, uint32_t n_ranks,
+                           const SpecOut& o, DevStatus* d_status, cudaStream_t st);
+void launch_pairs_spectrum(const DeviceInfo& di, const kmer_count_pair* d_pairs, uint64_t n, const SpecOut& o, DevStatus* d_status,
+                           cudaStream_t st);
 
 // count_part.cu --------------------------------------------------------------------------------
 struct PartitionPlan {
@@ -87,17 +104,19 @@ size_t partition_spill_bytes(const PartitionPlan& p);
 // DevStatus: n_overflow != 0 -> discard and recount (tier 3); n_failed / n_spill != 0 -> run tier 2.
 void launch_count_partition(const DeviceInfo& di, const ScanArgs& a, const PartitionPlan& p, unsigned long long* d_fill,
                             void* d_recs, void* d_spill, uint32_t* d_failed_ids, kmer_count_pair* d_pairs, uint64_t capacity,
-                            uint64_t* d_uniq, uint64_t uniq_capacity, cudaStream_t st, void (*mark)(void*, const char*), void* mark_arg);
+                            uint64_t* d_uniq, uint64_t uniq_capacity, cudaStream_t st, void (*mark)(void*, const char*), void* mark_arg,
+                            const SpecOut* spec = nullptr);
 // a.tile_begin/tile_end: the tiles this launch walks (a column that arrives in pieces); clear_fill = false appends to the regions
 void launch_partition(const DeviceInfo& di, const ScanArgs& a, const PartitionPlan& p, unsigned long long* d_fill,
                       void* d_recs, void* d_spill, cudaStream_t st, bool clear_fill = true);
 void launch_bucket_count(const DeviceInfo& di, const PartitionPlan& p, int k, const unsigned long long* d_fill,
                          const void* d_recs, void* d_spill, uint32_t* d_failed_ids, kmer_count_pair* d_pairs, uint64_t capacity,
                          uint64_t* d_uniq, uint64_t uniq_capacity, DevStatus* d_status, cudaStream_t st, uint32_t bucket_begin = 0,
-                         uint32_t bucket_end = 0);
+                         uint32_t bucket_end = 0, const SpecOut* spec = nullptr);
 // bucket_begin/bucket_end: the buckets this launch counts (0, 0: all) -- results can leave while later buckets are counted.
 // d_uniq != nullptr: split result format -- k-mers proven unique on chip are written as bare codes to d_uniq (counted in
-// DevStatus::n_unique), everything else as (k-mer, count) pairs
+// DevStatus::n_unique), everything else as (k-mer, count) pairs.  spec != nullptr: the spectrum result format instead (d_pairs,
+// d_uniq unused): every group the leaf counts is binned into spec->hist / spec->tail, nothing is written per group
 // Tier 2, stream-ordered: the device itself decides whether the failed buckets / spilled records need it (DevStatus::t2_mode);
 // all kernels are always launched and return at once when they are not needed.  d_slots: n_slots (a power of two) table slots;
 // if the failed k-mers do not fit, DevStatus::n_overflow is set (the caller recounts in kmer_cuda_dev_finish).
@@ -106,7 +125,7 @@ uint64_t tier2_table_slots(uint64_t n_kmers);
 void launch_partition_tier2(const DeviceInfo& di, const PartitionPlan& p, int k, const unsigned long long* d_fill,
                             const void* d_recs, const void* d_spill, const uint32_t* d_failed_ids, kmer_count_pair* d_slots,
                             uint64_t n_slots, kmer_count_pair* d_pairs, uint64_t capacity, DevStatus* d_status, cudaStream_t st,
-                            void (*mark)(void*, const char*), void* mark_arg);
+                            void (*mark)(void*, const char*), void* mark_arg, const SpecOut* spec = nullptr);
 // sharded counting, owner side: the coarse partitions received from every source GPU ([src][n_coarse][coarse_cap] records,
 // [src][n_coarse] fills) are split into this GPU's fine buckets (p: n_buckets = n_coarse << fine_shift, cap, spill list)
 // Source s's segments for THIS owner are src.recs[s] ([n_coarse][coarse_cap] records) and src.fill[s] ([n_coarse] fills): plain

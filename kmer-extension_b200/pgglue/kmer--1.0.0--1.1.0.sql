@@ -12,6 +12,16 @@ CREATE FUNCTION kmer_gpu_counts(dna[], integer)
     AS 'MODULE_PATHNAME', 'kmer_gpu_counts'
     LANGUAGE C IMMUTABLE STRICT PARALLEL SAFE;
 
+-- The k-mer abundance spectrum (count of counts) of that GROUP BY, binned on the GPU (no per-k-mer rows are materialised):
+--   SELECT * FROM kmer_gpu_count_spectrum(ARRAY(SELECT dna FROM reads), 21)
+--     ==  SELECT cnt AS count, count(*) AS kmers
+--         FROM (SELECT count(*) AS cnt FROM reads r, generate_kmers(r.dna, 21) AS g(kmer) GROUP BY g.kmer) s
+--         GROUP BY cnt ORDER BY cnt
+CREATE FUNCTION kmer_gpu_count_spectrum(dna[], integer)
+    RETURNS TABLE (count bigint, kmers bigint)
+    AS 'MODULE_PATHNAME', 'kmer_gpu_count_spectrum'
+    LANGUAGE C IMMUTABLE STRICT PARALLEL SAFE;
+
 -- equals / starts_with / contains over a column of k-mers against one constant (kmer.c:226-285):
 --   element i of the result:  op 0  kmer[i] = $2      op 1  kmer[i] ^@ $2      op 2  $2::qkmer @> kmer[i]
 CREATE FUNCTION kmer_gpu_match(kmer[], text, integer)

@@ -10,6 +10,8 @@
  *   kmer_gpu_match_datums()  : equals / starts_with / contains over a batch of `kmer` datums against one
  *                              constant, replacing per-row kmer_equals / kmer_starts_with / kmer_contains
  *                              calls (kmer.c:226-285).
+ *   kmer_gpu_spectrum_datums(): the k-mer abundance spectrum (count of counts) of that GROUP BY, binned on the GPU:
+ *                              (count, number of k-mers with that count) rows, ascending by count.
  *
  * Results are palloc'ed in the caller's memory context, exactly like the reference's functions
  * (kmer.c:92,124,341); `kmer` results carry the 1-byte short varlena header generate_kmers writes
@@ -35,6 +37,12 @@
  *   CREATE FUNCTION kmer_gpu_match(kmer[], text, integer) RETURNS SETOF boolean
  *       AS 'MODULE_PATHNAME', 'kmer_gpu_match' LANGUAGE C IMMUTABLE STRICT PARALLEL SAFE;
  *       -- element i: op 0 kmer[i] = $2 ; op 1 kmer[i] ^@ $2 ; op 2 $2::qkmer @> kmer[i]
+ *   CREATE FUNCTION kmer_gpu_count_spectrum(dna[], integer) RETURNS TABLE (count bigint, kmers bigint)
+ *       AS 'MODULE_PATHNAME', 'kmer_gpu_count_spectrum' LANGUAGE C IMMUTABLE STRICT PARALLEL SAFE;
+ *       -- SELECT * FROM kmer_gpu_count_spectrum(ARRAY(SELECT dna FROM reads), 21)
+ *       --   ==  SELECT cnt AS count, count(*) AS kmers
+ *       --       FROM (SELECT count(*) AS cnt FROM reads r, generate_kmers(r.dna, 21) AS g(kmer) GROUP BY g.kmer) s
+ *       --       GROUP BY cnt ORDER BY cnt
  */
 
 
@@ -161,6 +169,87 @@ kmer_gpu_count_datums(struct varlena **dnas, uint64_t n, int k, struct varlena *
 	*n_groups = d;
 }
 
+/* counts below this are binned by the library; the (rare) groups above it come back whole and are folded in here */
+#define KMER_GPU_SPECTRUM_HIST_LEN 65536
+
+static int
+cmp_u64(const void *a, const void *b)
+{
+	uint64_t x = *(const uint64_t *) a, y = *(const uint64_t *) b;
+
+	return x < y ? -1 : x > y;
+}
+
+/*
+ * dnas[0..n) as for kmer_gpu_count_datums.  On return (*counts)[i], (*kmers)[i] for i < *n_out are the rows of the spectrum:
+ * every count that occurs, ascending, and the number of distinct k-mers with exactly that count.
+ */
+void
+kmer_gpu_spectrum_datums(struct varlena **dnas, uint64_t n, int k, int64_t **counts, int64_t **kmers, uint64_t *n_out)
+{
+	kmer_cuda_ctx *ctx = kmer_gpu_context();
+	uint64_t *off = (uint64_t *) palloc((n + 1) * sizeof(uint64_t));
+	uint64_t total = 0, i, n_tail = 0, n_kmers = 0, m = 0;
+	uint64_t *hist = NULL;
+	kmer_count_pair *tail = NULL;
+	char *flat;
+
+	off[0] = 0;
+	for (i = 0; i < n; i++)
+	{
+		total += (uint64_t) VARSIZE_ANY_EXHDR(dnas[i]);
+		off[i + 1] = total;
+	}
+	flat = (char *) palloc(total + 16);
+	for (i = 0; i < n; i++)
+		memcpy(flat + off[i], VARDATA_ANY(dnas[i]), (size_t) (off[i + 1] - off[i]));
+	if (kmer_cuda_submit_count_spectrum(ctx, flat, off, n, k, KMER_GPU_SPECTRUM_HIST_LEN, &hist, &tail, &n_tail, &n_kmers) != KMER_OK)
+		kmer_gpu_raise(kmer_cuda_last_error(ctx));
+
+	void *volatile r_hist = hist, *volatile r_tail = tail; /* pinned library buffers: released on every path */
+
+	PG_TRY();
+	{
+		uint64_t *tc = (uint64_t *) palloc((n_tail ? n_tail : 1) * sizeof(uint64_t));
+		uint64_t rows = n_tail;
+
+		for (i = 1; i < KMER_GPU_SPECTRUM_HIST_LEN; i++)
+			rows += hist[i] != 0;
+		*counts = (int64_t *) palloc((rows ? rows : 1) * sizeof(int64_t));
+		*kmers = (int64_t *) palloc((rows ? rows : 1) * sizeof(int64_t));
+		for (i = 1; i < KMER_GPU_SPECTRUM_HIST_LEN; i++)
+			if (hist[i])
+			{
+				(*counts)[m] = (int64_t) i;
+				(*kmers)[m++] = (int64_t) hist[i];
+			}
+		/* the tail: one group per high-copy k-mer, every count >= KMER_GPU_SPECTRUM_HIST_LEN -- sorted and grouped by count */
+		for (i = 0; i < n_tail; i++)
+			tc[i] = tail[i].count;
+		qsort(tc, n_tail, sizeof(uint64_t), cmp_u64);
+		for (i = 0; i < n_tail; i++)
+		{
+			if (i && tc[i] == tc[i - 1])
+				(*kmers)[m - 1]++;
+			else
+			{
+				(*counts)[m] = (int64_t) tc[i];
+				(*kmers)[m++] = 1;
+			}
+		}
+	}
+	PG_CATCH();
+	{
+		kmer_cuda_release(ctx, r_hist);
+		kmer_cuda_release(ctx, r_tail);
+		PG_RE_THROW();
+	}
+	PG_END_TRY();
+	kmer_cuda_release(ctx, r_hist);
+	kmer_cuda_release(ctx, r_tail);
+	*n_out = m;
+}
+
 /*
  * op: KMER_OP_EQUALS (kmer = const), KMER_OP_STARTS_WITH (kmer ^@ const), KMER_OP_CONTAINS (const::qkmer @> kmer).
  * kmers[0..n) are `kmer` datums of any lengths 0..32; result[i] is the boolean the reference returns.
@@ -258,6 +347,68 @@ kmer_gpu_counts(PG_FUNCTION_ARGS)
 
 		values[0] = PointerGetDatum(st->kmers[funcctx->call_cntr]);
 		values[1] = Int64GetDatum(st->counts[funcctx->call_cntr]);
+		tuple = HeapTupleGetDatum(heap_form_tuple(st->tupdesc, values, isnull)); /* before SRF_RETURN_NEXT bumps call_cntr */
+		SRF_RETURN_NEXT(funcctx, tuple);
+	}
+	SRF_RETURN_DONE(funcctx);
+}
+
+typedef struct SpectrumState
+{
+	int64_t *counts;
+	int64_t *kmers;
+	TupleDesc tupdesc;
+} SpectrumState;
+
+PG_FUNCTION_INFO_V1(kmer_gpu_count_spectrum);
+/*
+ * kmer_gpu_count_spectrum(dna[], k) -> setof (count bigint, kmers bigint), ascending by count: the abundance spectrum of
+ * kmer_gpu_counts(dna[], k), computed without materialising the groups.  The batch is counted on the first call.
+ */
+Datum
+kmer_gpu_count_spectrum(PG_FUNCTION_ARGS)
+{
+	FuncCallContext *funcctx;
+	SpectrumState *st;
+
+	if (SRF_IS_FIRSTCALL())
+	{
+		MemoryContext oldcontext;
+		ArrayType *arr = PG_GETARG_ARRAYTYPE_P(0);
+		int32 k = PG_GETARG_INT32(1);
+		Datum *elems;
+		bool *nulls;
+		int n, i, m = 0;
+		struct varlena **dnas;
+		uint64_t n_rows = 0;
+		TupleDesc tupdesc;
+
+		funcctx = SRF_FIRSTCALL_INIT();
+		oldcontext = MemoryContextSwitchTo(funcctx->multi_call_memory_ctx);
+		if (get_call_result_type(fcinfo, NULL, &tupdesc) != TYPEFUNC_COMPOSITE)
+			ereport(ERROR, (errcode(ERRCODE_INTERNAL_ERROR), errmsg("kmer_gpu_count_spectrum must return a composite type")));
+		deconstruct_array(arr, ARR_ELEMTYPE(arr), -1, false, 'i', &elems, &nulls, &n);
+		dnas = (struct varlena **) palloc((n ? n : 1) * sizeof(struct varlena *));
+		for (i = 0; i < n; i++)
+			if (!nulls || !nulls[i]) /* generate_kmers is STRICT: a NULL dna yields no rows */
+				dnas[m++] = PG_DETOAST_DATUM(elems[i]);
+		st = (SpectrumState *) palloc(sizeof(SpectrumState));
+		st->tupdesc = BlessTupleDesc(tupdesc);
+		kmer_gpu_spectrum_datums(dnas, (uint64_t) m, k, &st->counts, &st->kmers, &n_rows);
+		funcctx->max_calls = n_rows;
+		funcctx->user_fctx = st;
+		MemoryContextSwitchTo(oldcontext);
+	}
+	funcctx = SRF_PERCALL_SETUP();
+	st = (SpectrumState *) funcctx->user_fctx;
+	if (funcctx->call_cntr < funcctx->max_calls)
+	{
+		Datum values[2];
+		bool isnull[2] = {false, false};
+		Datum tuple;
+
+		values[0] = Int64GetDatum(st->counts[funcctx->call_cntr]);
+		values[1] = Int64GetDatum(st->kmers[funcctx->call_cntr]);
 		tuple = HeapTupleGetDatum(heap_form_tuple(st->tupdesc, values, isnull)); /* before SRF_RETURN_NEXT bumps call_cntr */
 		SRF_RETURN_NEXT(funcctx, tuple);
 	}

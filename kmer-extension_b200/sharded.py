@@ -169,6 +169,27 @@ class ShardedCounter:
             total_kmers = self._allreduce_int(local_kmers)
         if k <= 13:
             return self._count_dense(d_seq, n_bases, d_off, n_rows, k, d_pairs, total_kmers)
+
+        def owner_count(plan, pst, recv_recs, recv_fill, recs_bytes):
+            if pst is not None:
+                rb, bpr = plan.recs_bytes_per_peer, plan.buckets_per_rank
+                eng.dev_shard_count_peers(plan, [a + self.rank * rb for a in pst["addr"]],
+                                          [a + recs_bytes + self.rank * bpr * 8 for a in pst["addr"]], d_uniq, d_pairs)
+            elif d_uniq is not None:
+                eng.dev_shard_count_split(plan, recv_recs, recv_fill, d_uniq, d_pairs)
+            else:
+                eng.dev_shard_count(plan, recv_recs, recv_fill, d_pairs)
+        r = self._exchange_and_count(d_seq, n_bases, d_off, n_rows, k, total_kmers, owner_count)
+        if r is None:                     # skewed input: some segment or spill list ran out of room -- exact fallback, all ranks together
+            return self._count_fallback(d_seq, n_bases, d_off, n_rows, k, d_pairs, total_kmers)
+        return int(r.n_distinct), int(r.n_kmers), {"tier2_kmers": int(r.n_tier2), "plan": self.last_plan,
+                                                  "n_unique": int(getattr(r, "n_unique", 0)), "fallback": False}
+
+    def _exchange_and_count(self, d_seq, n_bases, d_off, n_rows, k, total_kmers, owner_count):
+        """The minimizer exchange (k >= 14) and this rank's owner count, owner_count(plan, pull state or None, recv_recs,
+        recv_fill, recs_bytes) -- one of the library's dev_shard_count* calls.  Returns the count's dev_finish result, or None
+        when some rank ran out of room (KMER_ERR_CAPACITY): every rank then takes the exact fallback together."""
+        eng = self.eng
         # chunks=2 partitions the rows in two pieces and exchanges the first on a side stream while the second is being
         # partitioned.  Measured on 2xB200 it LOSES (18.8 vs 17.9 ms/step: two launches and host round trips per step, and
         # the exchange slows the partition kernel it runs beside), so it is opt-in.
@@ -268,14 +289,7 @@ class ShardedCounter:
         r = None
         if exc is None:
             try:
-                if pull:
-                    rb, bpr = plan.recs_bytes_per_peer, plan.buckets_per_rank
-                    eng.dev_shard_count_peers(plan, [a + self.rank * rb for a in pst["addr"]],
-                                              [a + recs_bytes + self.rank * bpr * 8 for a in pst["addr"]], d_uniq, d_pairs)
-                elif d_uniq is not None:
-                    eng.dev_shard_count_split(plan, recv_recs, recv_fill, d_uniq, d_pairs)
-                else:
-                    eng.dev_shard_count(plan, recv_recs, recv_fill, d_pairs)
+                owner_count(plan, pst if pull else None, recv_recs, recv_fill, recs_bytes)
                 r = eng.dev_finish()
             except Exception as e:        # no rank may be left waiting in a collective
                 exc = e
@@ -291,14 +305,78 @@ class ShardedCounter:
             if code == 2:
                 raise exc
             raise RuntimeError("sharded count aborted: another rank reported an input error")
-        if n_capacity:                    # skewed input: some segment or spill list ran out of room -- exact fallback, all ranks together
-            return self._count_fallback(d_seq, n_bases, d_off, n_rows, k, d_pairs, total_kmers)
+        if n_capacity:
+            return None
         phases += self._phases()
         self.last_phases = phases
         if counted != total_kmers:
             raise RuntimeError(f"sharded count lost k-mers: counted {counted}, expected {total_kmers}")
-        return int(r.n_distinct), int(r.n_kmers), {"tier2_kmers": int(r.n_tier2), "plan": plan,
-                                                  "n_unique": int(getattr(r, "n_unique", 0)), "fallback": False}
+        return r
+
+    def spectrum(self, d_seq, n_bases: int, d_off, n_rows: int, k: int, hist_len: int = 65536, total_kmers: int | None = None):
+        """The abundance spectrum (count of counts) of this rank's rows together with all other ranks' rows; collective.
+
+        Returns (hist, tail, info), the SAME on every rank: hist int64 [hist_len] -- hist[c] = k-mers counted exactly c times --
+        and tail int64 [n, 2], the (code, count) groups with count >= hist_len, ranks' tails in rank order.  Every owner bins its
+        own groups (disjoint across ranks), then one all-reduce sums the histograms and an all-gather joins the tails."""
+        eng = self.eng
+        if total_kmers is None:
+            total_kmers = self._allreduce_int(eng.max_kmers(n_bases, n_rows, k))
+        hist = self._buf("spec_hist", hist_len * 8, torch.int64)
+        tail = self._buf("spec_tail", max(total_kmers // hist_len, 1) * 16, torch.int64).view(-1, 2)
+        info = {"plan": None, "fallback": False, "tier2_kmers": 0}
+        if k <= 13:
+            owned = self._buf("spec_pairs", ((1 << (2 * k)) + self.world - 1) // self.world * 16, torch.int64).view(-1, 2)
+            nd, _, _ = self._count_dense(d_seq, n_bases, d_off, n_rows, k, owned, total_kmers)
+            n_tail = self._pairs_spectrum(owned, nd, hist, tail)
+        else:
+            def owner_count(plan, pst, recv_recs, recv_fill, recs_bytes):
+                rb, bpr = plan.recs_bytes_per_peer, plan.buckets_per_rank
+                if pst is not None:
+                    src_r = [a + self.rank * rb for a in pst["addr"]]
+                    src_f = [a + recs_bytes + self.rank * bpr * 8 for a in pst["addr"]]
+                else:                         # the receive buffers: source s's segments at s * recs_bytes_per_peer
+                    n_src = recv_fill.numel() // bpr
+                    src_r = [recv_recs.data_ptr() + s * rb for s in range(n_src)]
+                    src_f = [recv_fill.data_ptr() + s * bpr * 8 for s in range(n_src)]
+                eng.dev_shard_count_spectrum(plan, src_r, src_f, hist, tail)
+            r = self._exchange_and_count(d_seq, n_bases, d_off, n_rows, k, total_kmers, owner_count)
+            if r is None:                 # the exact fallback: the owners' merged tables, then their spectrum
+                owned = self._buf("spec_pairs", (int(total_kmers / self.world * 1.3) + 65536) * 16, torch.int64).view(-1, 2)
+                nd, _, info = self._count_fallback(d_seq, n_bases, d_off, n_rows, k, owned, total_kmers)
+                n_tail = self._pairs_spectrum(owned, nd, hist, tail)
+            else:
+                n_tail = int(r.n_distinct)
+                info = {"plan": self.last_plan, "fallback": False, "tier2_kmers": int(r.n_tier2)}
+        hist_all, tail_all = self._combine_spectrum(hist, tail[:n_tail])
+        return hist_all, tail_all, info
+
+    def _pairs_spectrum(self, pairs, n, hist, tail) -> int:
+        exc, r = None, None
+        try:
+            self.eng.dev_pairs_spectrum(pairs, n, hist, tail)
+            r = self.eng.dev_finish()
+        except Exception as e:
+            exc = e
+        if self._agree(exc) or exc is not None:
+            raise exc if exc is not None else RuntimeError("sharded spectrum aborted: another rank's tail buffer is too small")
+        return int(r.n_distinct)
+
+    def _combine_spectrum(self, hist, tail):
+        """The owners' spectra -> the job's: histograms summed, tails gathered (sizes first), on every rank."""
+        hist = hist.clone()
+        if self.world == 1:
+            return hist, tail.clone()
+        dist.all_reduce(hist, op=dist.ReduceOp.SUM, group=self.group)
+        n = torch.tensor([tail.shape[0]], dtype=torch.int64, device=self.device)
+        sizes = [torch.zeros_like(n) for _ in range(self.world)]
+        dist.all_gather(sizes, n, group=self.group)
+        sizes = [int(x.item()) for x in sizes]
+        pad = torch.zeros((max(max(sizes), 1), 2), dtype=torch.int64, device=self.device)
+        pad[:tail.shape[0]] = tail
+        parts = [torch.empty_like(pad) for _ in range(self.world)]
+        dist.all_gather(parts, pad, group=self.group)
+        return hist, torch.cat([p[:m] for p, m in zip(parts, sizes)])
 
     def _count_fallback(self, d_seq, n_bases, d_off, n_rows, k, d_pairs, total_kmers):
         """Exact on ANY input (HashAggregate never refuses rows, kmer-tests.sql:1208-1213): every rank counts its own rows with
