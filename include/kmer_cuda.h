@@ -151,6 +151,26 @@ int kmer_cuda_submit_count_spectrum(kmer_cuda_ctx *ctx, const char *seq, const u
 									uint64_t hist_len, uint64_t **hist, kmer_count_pair **tail, uint64_t *n_tail,
 									uint64_t *n_kmers);
 
+/* Canonical k-mer counting: a k-mer and its reverse complement are one group (what `jellyfish count -C`, KMC and Gerbil count by
+ * default, and the spectrum GenomeScope expects: reads come from both strands).  rc(x) complements every base (a<->t, c<->g) and
+ * reverses their order; canon(x) = min(x, rc(x)), which is also the smaller of the two lower-case texts.  One group per value of
+ * canon over all windows of all rows, counted over windows of either orientation; equal to the stock SQL
+ *   SELECT least(g.kmer::text COLLATE "C", reverse(translate(g.kmer::text, 'acgt', 'tgca')))::kmer AS kmer, count(*)
+ *   FROM reads r, generate_kmers(r.dna, k) AS g(kmer) GROUP BY 1
+ * Errors and the offending row are exactly those of kmer_cuda_submit_count.  Every code returned is canonical; at k = 32 the
+ * all-t and all-a windows are one group with code 0.  The strand-specific calls are unchanged (they are the reference's
+ * contract); canonical counting is a separate set of entry points, never a mode left on a context.  Not covered: sharded
+ * counting, the packed format, extract.
+ * uniq_codes == NULL: every group in (*pairs)[0..*n_pairs) (kmer_cuda_submit_count's format); else the split format of
+ * kmer_cuda_submit_count_split.  Results are released with kmer_cuda_release(). */
+int kmer_cuda_submit_count_canonical(kmer_cuda_ctx *ctx, const char *seq, const uint64_t *row_off, uint64_t n_rows, int k,
+									 uint64_t **uniq_codes, uint64_t *n_unique, kmer_count_pair **pairs, uint64_t *n_pairs,
+									 uint64_t *n_kmers);
+/* The abundance spectrum of the canonical GROUP BY: the contract of kmer_cuda_submit_count_spectrum. */
+int kmer_cuda_submit_count_canonical_spectrum(kmer_cuda_ctx *ctx, const char *seq, const uint64_t *row_off, uint64_t n_rows,
+											  int k, uint64_t hist_len, uint64_t **hist, kmer_count_pair **tail, uint64_t *n_tail,
+											  uint64_t *n_kmers);
+
 /* Replaces per-row calls of kmer_equals / kmer_starts_with[_op] / kmer_contains / kmer_containing
  * (kmer.c:226-285) over a column of m k-mers against n_consts constants given as text:
  *   KMER_OP_EQUALS, KMER_OP_STARTS_WITH : constants are kmer literals   (kmer_in rules, kmer.c:109-129)
@@ -218,6 +238,16 @@ int kmer_cuda_dev_count_split(kmer_cuda_ctx *ctx, const char *d_seq, uint64_t n_
 int kmer_cuda_dev_count_spectrum(kmer_cuda_ctx *ctx, const char *d_seq, uint64_t n_bases, const uint64_t *d_row_off,
 								 uint64_t n_rows, int k, uint64_t *d_hist, uint64_t hist_len, kmer_count_pair *d_tail,
 								 uint64_t tail_capacity, int algo, void *stream);
+/* Canonical counting (see kmer_cuda_submit_count_canonical) on device buffers.  d_uniq == NULL: every group as a pair in d_pairs
+ * (kmer_cuda_dev_count's format); else the split format of kmer_cuda_dev_count_split.  algo as kmer_cuda_dev_count, except that
+ * 4 runs as 3 (the two-pass partition has no canonical minimizer). */
+int kmer_cuda_dev_count_canonical(kmer_cuda_ctx *ctx, const char *d_seq, uint64_t n_bases, const uint64_t *d_row_off,
+								  uint64_t n_rows, int k, uint64_t *d_uniq, uint64_t uniq_capacity, kmer_count_pair *d_pairs,
+								  uint64_t pairs_capacity, int algo, void *stream);
+/* The spectrum of the canonical GROUP BY: the arguments, outputs and finish() report of kmer_cuda_dev_count_spectrum. */
+int kmer_cuda_dev_count_canonical_spectrum(kmer_cuda_ctx *ctx, const char *d_seq, uint64_t n_bases, const uint64_t *d_row_off,
+										   uint64_t n_rows, int k, uint64_t *d_hist, uint64_t hist_len, kmer_count_pair *d_tail,
+										   uint64_t tail_capacity, int algo, void *stream);
 /* The spectrum of a (k-mer, count) table already in HBM, d_pairs[0..n): same outputs and finish() report. */
 int kmer_cuda_dev_pairs_spectrum(kmer_cuda_ctx *ctx, const kmer_count_pair *d_pairs, uint64_t n, uint64_t *d_hist,
 								 uint64_t hist_len, kmer_count_pair *d_tail, uint64_t tail_capacity, void *stream);

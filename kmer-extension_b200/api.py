@@ -45,6 +45,8 @@ ABI_SYMBOLS = [
     "kmer_cuda_init_multi", "kmer_cuda_shutdown_multi", "kmer_cuda_multi_device_count", "kmer_cuda_multi_last_error",
     "kmer_cuda_multi_submit_count", "kmer_cuda_multi_release", "kmer_cuda_dev_pack_codes", "kmer_cuda_multi_submit_match", "kmer_cuda_dev_synth_reads",
     "kmer_cuda_dev_count_spectrum", "kmer_cuda_dev_shard_count_spectrum", "kmer_cuda_dev_pairs_spectrum", "kmer_cuda_submit_count_spectrum",
+    "kmer_cuda_dev_count_canonical", "kmer_cuda_dev_count_canonical_spectrum", "kmer_cuda_submit_count_canonical",
+    "kmer_cuda_submit_count_canonical_spectrum",
 ]
 
 
@@ -130,6 +132,10 @@ def load_library(path: Path = LIB_PATH) -> C.CDLL:
     L.kmer_cuda_dev_shard_count_spectrum.argtypes = [vp, C.POINTER(KmerShardPlan), C.POINTER(vp), C.POINTER(vp), vp, u64, vp, u64, vp]
     L.kmer_cuda_dev_pairs_spectrum.argtypes = [vp, vp, u64, vp, u64, vp, u64, vp]
     L.kmer_cuda_submit_count_spectrum.argtypes = [vp, vp, vp, u64, i32, u64, C.POINTER(vp), C.POINTER(vp), u64p, u64p]
+    L.kmer_cuda_dev_count_canonical.argtypes = [vp, vp, u64, vp, u64, i32, vp, u64, vp, u64, i32, vp]
+    L.kmer_cuda_dev_count_canonical_spectrum.argtypes = [vp, vp, u64, vp, u64, i32, vp, u64, vp, u64, i32, vp]
+    L.kmer_cuda_submit_count_canonical.argtypes = [vp, vp, vp, u64, i32, C.POINTER(vp), u64p, C.POINTER(vp), u64p, u64p]
+    L.kmer_cuda_submit_count_canonical_spectrum.argtypes = [vp, vp, vp, u64, i32, u64, C.POINTER(vp), C.POINTER(vp), u64p, u64p]
     return L
 
 
@@ -144,6 +150,21 @@ def _flat(rows_or_flat, off=None):
     if bs:
         o[1:] = np.cumsum([len(b) for b in bs], dtype=np.uint64)
     return np.frombuffer(b"".join(bs), dtype=np.uint8), o
+
+
+def revcomp_codes(codes, k: int) -> np.ndarray:
+    """Codes of the reverse complements (a<->t, c<->g, order reversed) of k-mer codes (numpy, uint64)."""
+    x = ~np.asarray(codes, dtype=np.uint64)
+    r = np.zeros_like(x)
+    for i in range(k):                                          # base i (from the first) becomes base k-1-i
+        r |= ((x >> np.uint64(2 * (k - 1 - i))) & np.uint64(3)) << np.uint64(2 * i)
+    return r
+
+
+def canonical_codes(codes, k: int) -> np.ndarray:
+    """min(code, reverse complement): the group key of canonical counting."""
+    c = np.asarray(codes, dtype=np.uint64)
+    return np.minimum(c, revcomp_codes(c, k))
 
 
 def spectrum_rows(hist, tail):
@@ -230,21 +251,27 @@ class KmerCuda:
                                                       C.byref(codes), C.byref(n)))
         return self._take(codes, n.value * 8, np.uint64)
 
-    def count_kmers(self, rows_or_flat, k: int, off=None):
-        """GROUP BY kmer / count(*) -> (codes[D] uint64, counts[D] uint64, n_kmers); order unspecified."""
+    def count_kmers(self, rows_or_flat, k: int, off=None, canonical: bool = False):
+        """GROUP BY kmer / count(*) -> (codes[D] uint64, counts[D] uint64, n_kmers); order unspecified.  canonical: a k-mer and
+        its reverse complement are one group, keyed by canonical_codes()."""
         f, o = _flat(rows_or_flat, off)
         pairs, d, n = C.c_void_p(), C.c_uint64(), C.c_uint64()
-        self._check(self.lib.kmer_cuda_submit_count(self.ctx, f.ctypes.data, o.ctypes.data, len(o) - 1, k,
-                                                    C.byref(pairs), C.byref(d), C.byref(n)))
+        if canonical:
+            self._check(self.lib.kmer_cuda_submit_count_canonical(self.ctx, f.ctypes.data, o.ctypes.data, len(o) - 1, k, None, None,
+                                                                  C.byref(pairs), C.byref(d), C.byref(n)))
+        else:
+            self._check(self.lib.kmer_cuda_submit_count(self.ctx, f.ctypes.data, o.ctypes.data, len(o) - 1, k,
+                                                        C.byref(pairs), C.byref(d), C.byref(n)))
         a = self._take(pairs, d.value * 16, np.uint64).reshape(-1, 2)
         return a[:, 0].copy(), a[:, 1].copy(), int(n.value)
 
-    def count_kmers_split(self, rows_or_flat, k: int, off=None):
+    def count_kmers_split(self, rows_or_flat, k: int, off=None, canonical: bool = False):
         """The same GROUP BY in the split format -> (unique codes[U], codes[P], counts[P], n_kmers)."""
         f, o = _flat(rows_or_flat, off)
         uq, nu, pairs, npairs, n = C.c_void_p(), C.c_uint64(), C.c_void_p(), C.c_uint64(), C.c_uint64()
-        self._check(self.lib.kmer_cuda_submit_count_split(self.ctx, f.ctypes.data, o.ctypes.data, len(o) - 1, k, C.byref(uq),
-                                                          C.byref(nu), C.byref(pairs), C.byref(npairs), C.byref(n)))
+        fn = self.lib.kmer_cuda_submit_count_canonical if canonical else self.lib.kmer_cuda_submit_count_split
+        self._check(fn(self.ctx, f.ctypes.data, o.ctypes.data, len(o) - 1, k, C.byref(uq), C.byref(nu), C.byref(pairs),
+                       C.byref(npairs), C.byref(n)))
         u = self._take(uq, nu.value * 8, np.uint64)
         a = self._take(pairs, npairs.value * 16, np.uint64).reshape(-1, 2)
         return u.copy(), a[:, 0].copy(), a[:, 1].copy(), int(n.value)
@@ -262,13 +289,14 @@ class KmerCuda:
         a = self._take(pairs, npairs.value * 16, np.uint64).reshape(-1, 2)
         return u, a[:, 0].copy(), a[:, 1].copy(), int(n.value), int(nb.value)
 
-    def count_spectrum(self, rows_or_flat, k: int, off=None, hist_len: int = 65536):
+    def count_spectrum(self, rows_or_flat, k: int, off=None, hist_len: int = 65536, canonical: bool = False):
         """Abundance spectrum of the GROUP BY -> (hist[hist_len] uint64, tail [n, 2] uint64 (code, count) of the groups with
         count >= hist_len, order unspecified); spectrum_rows(hist, tail) is the SQL relation."""
         f, o = _flat(rows_or_flat, off)
         hist, tail, nt, n = C.c_void_p(), C.c_void_p(), C.c_uint64(), C.c_uint64()
-        self._check(self.lib.kmer_cuda_submit_count_spectrum(self.ctx, f.ctypes.data, o.ctypes.data, len(o) - 1, k, hist_len,
-                                                             C.byref(hist), C.byref(tail), C.byref(nt), C.byref(n)))
+        fn = self.lib.kmer_cuda_submit_count_canonical_spectrum if canonical else self.lib.kmer_cuda_submit_count_spectrum
+        self._check(fn(self.ctx, f.ctypes.data, o.ctypes.data, len(o) - 1, k, hist_len, C.byref(hist), C.byref(tail), C.byref(nt),
+                       C.byref(n)))
         h = self._take(hist, hist_len * 8, np.uint64)
         t = self._take(tail, nt.value * 16, np.uint64).reshape(-1, 2)
         return h, t
@@ -344,23 +372,34 @@ class KmerCuda:
         self._check(self.lib.kmer_cuda_dev_extract(self.ctx, d_seq.data_ptr(), n_bases, d_off.data_ptr(), n_rows, k,
                                                    d_codes.data_ptr(), d_codes.numel(), self._stream_ptr(stream)))
 
-    def dev_count(self, d_seq, n_bases: int, d_off, n_rows: int, k: int, d_pairs, algo: int = ALGO_AUTO, stream=None):
-        """d_pairs: int64/uint64 tensor [capacity, 2]."""
+    def dev_count(self, d_seq, n_bases: int, d_off, n_rows: int, k: int, d_pairs, algo: int = ALGO_AUTO, stream=None,
+                  canonical: bool = False):
+        """d_pairs: int64/uint64 tensor [capacity, 2].  canonical: canonical k-mers (ALGO_TWO_PASS runs as ALGO_PARTITION)."""
+        if canonical:
+            self._check(self.lib.kmer_cuda_dev_count_canonical(self.ctx, d_seq.data_ptr(), n_bases, d_off.data_ptr(), n_rows, k, None, 0,
+                                                               d_pairs.data_ptr(), d_pairs.numel() // 2, algo, self._stream_ptr(stream)))
+            return
         self._check(self.lib.kmer_cuda_dev_count(self.ctx, d_seq.data_ptr(), n_bases, d_off.data_ptr(), n_rows, k,
                                                  d_pairs.data_ptr(), d_pairs.numel() // 2, algo, self._stream_ptr(stream)))
 
-    def dev_count_split(self, d_seq, n_bases: int, d_off, n_rows: int, k: int, d_uniq, d_pairs, stream=None):
+    def dev_count_split(self, d_seq, n_bases: int, d_off, n_rows: int, k: int, d_uniq, d_pairs, stream=None, canonical: bool = False):
         """d_uniq: uint64/int64 tensor [capacity]; d_pairs: [capacity, 2]."""
+        if canonical:
+            self._check(self.lib.kmer_cuda_dev_count_canonical(self.ctx, d_seq.data_ptr(), n_bases, d_off.data_ptr(), n_rows, k,
+                                                               d_uniq.data_ptr(), d_uniq.numel(), d_pairs.data_ptr(), d_pairs.numel() // 2,
+                                                               ALGO_AUTO, self._stream_ptr(stream)))
+            return
         self._check(self.lib.kmer_cuda_dev_count_split(self.ctx, d_seq.data_ptr(), n_bases, d_off.data_ptr(), n_rows, k,
                                                        d_uniq.data_ptr(), d_uniq.numel(), d_pairs.data_ptr(), d_pairs.numel() // 2,
                                                        self._stream_ptr(stream)))
 
-    def dev_count_spectrum(self, d_seq, n_bases: int, d_off, n_rows: int, k: int, d_hist, d_tail, algo: int = ALGO_AUTO, stream=None):
+    def dev_count_spectrum(self, d_seq, n_bases: int, d_off, n_rows: int, k: int, d_hist, d_tail, algo: int = ALGO_AUTO, stream=None,
+                           canonical: bool = False):
         """Spectrum result format: d_hist uint64/int64 [hist_len] (overwritten whole), d_tail [tail_capacity, 2] gets the groups
         with count >= hist_len; dev_finish().n_distinct = tail entries written."""
-        self._check(self.lib.kmer_cuda_dev_count_spectrum(self.ctx, d_seq.data_ptr(), n_bases, d_off.data_ptr(), n_rows, k,
-                                                          d_hist.data_ptr(), d_hist.numel(), d_tail.data_ptr(), d_tail.shape[0], algo,
-                                                          self._stream_ptr(stream)))
+        fn = self.lib.kmer_cuda_dev_count_canonical_spectrum if canonical else self.lib.kmer_cuda_dev_count_spectrum
+        self._check(fn(self.ctx, d_seq.data_ptr(), n_bases, d_off.data_ptr(), n_rows, k, d_hist.data_ptr(), d_hist.numel(),
+                       d_tail.data_ptr(), d_tail.shape[0], algo, self._stream_ptr(stream)))
 
     def dev_pairs_spectrum(self, d_pairs, n: int, d_hist, d_tail, stream=None):
         """The spectrum of the (code, count) table d_pairs[:n] (same outputs as dev_count_spectrum)."""

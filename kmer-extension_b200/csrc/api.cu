@@ -63,6 +63,7 @@ struct kmer_cuda_ctx {
     uint64_t p_pairs_cap = 0;
     // ... or, in the spectrum result format, re-zeroes the histogram and rebins into it (the tail cursor is DevStatus::n_distinct)
     bool p_spectrum = false;
+    bool p_canonical = false;     // ... and counts canonical k-mers (kmer_cuda_*_count_canonical*)
     uint64_t* p_hist = nullptr;
     uint64_t p_hist_len = 0;
     kmer_count_pair* p_tail = nullptr;
@@ -443,6 +444,7 @@ static int begin_op(kmer_cuda_ctx* c, cudaStream_t st, bool keep_input_findings 
     c->pending = OP_NONE;
     c->p_recountable = false;
     c->p_spectrum = false;
+    c->p_canonical = false;
     return KMER_OK;
 }
 
@@ -524,10 +526,10 @@ static int spectrum_begin(kmer_cuda_ctx* c, const SpecOut& o, cudaStream_t st) {
 }
 
 // d_uniq != nullptr: split result format (see kmer_cuda_dev_count_split); spec != nullptr: spectrum result format
-// (kmer_cuda_dev_count_spectrum; d_pairs / d_uniq unused)
+// (kmer_cuda_dev_count_spectrum; d_pairs / d_uniq unused); canon: canonical k-mers (kmer_cuda_dev_count_canonical; algo 4 runs as 3)
 static int dev_count_impl(kmer_cuda_ctx* c, const char* d_seq, uint64_t n_bases, const uint64_t* d_row_off, uint64_t n_rows, int k,
                           kmer_count_pair* d_pairs, uint64_t pairs_capacity, uint64_t* d_uniq, uint64_t uniq_capacity, int algo,
-                          void* stream, const SpecOut* spec = nullptr) {
+                          void* stream, const SpecOut* spec = nullptr, bool canon = false) {
     if (!c) return KMER_ERR_BAD_ARGUMENT;
     cudaStream_t st = pick_stream(c, stream);
     int rc = begin_op(c, st);
@@ -547,11 +549,12 @@ static int dev_count_impl(kmer_cuda_ctx* c, const char* d_seq, uint64_t n_bases,
     rc = prepare_rows(c, d_row_off, n_bases, n_rows, k, st, &a, d_seq);
     if (rc) return rc;
     if (algo == 0) algo = (k <= 13) ? 1 : 3;
+    if (canon && algo == 4) algo = 3;                                   // the two-pass scatter has no canonical minimizer
     c->last_overflow = 0;
     c->last_tier2 = 0;
     if (algo == 3 || algo == 4) {
         if (k < 14) return bad_arg(c, "minimizer-partition counting needs k >= 14");
-        PartitionPlan plan = make_partition_plan(c->p_expected_kmers, k);
+        PartitionPlan plan = make_partition_plan(c->p_expected_kmers, k, canon);
         ScatterPlan sp{};
         // algo 4: the two write-combining passes of scatter.cuh instead of partition_kernel's scattered record stores.  Measured
         // (1 GB, k=21): 4.2 + 2.4 ms against 6.5 ms -- no gain yet (both passes are instruction bound), so it is opt-in.
@@ -576,15 +579,16 @@ static int dev_count_impl(kmer_cuda_ctx* c, const char* d_seq, uint64_t n_bases,
             c->launches += 3;
         } else {
             launch_count_partition(c->di, a, plan, (unsigned long long*)c->fill.p, c->recs.p, c->spill.p, (uint32_t*)c->failed.p,
-                                   d_pairs, pairs_capacity, d_uniq, uniq_capacity, st, mark_cb, &ma, spec);
+                                   d_pairs, pairs_capacity, d_uniq, uniq_capacity, st, mark_cb, &ma, spec, canon);
             c->launches += 2;
         }
         // Tier 2 (buckets that did not fit on chip, spilled records) is decided and run by the device: nothing here waits
         // for the GPU.  Only a batch that overflows even that (DevStatus::n_overflow) is recounted, by kmer_cuda_dev_finish.
         launch_partition_tier2(c->di, plan, k, (const unsigned long long*)c->fill.p, c->recs.p, c->spill.p, (const uint32_t*)c->failed.p,
-                               (kmer_count_pair*)c->table.p, t2_slots, d_pairs, pairs_capacity, c->d_status, st, mark_cb, &ma, spec);
+                               (kmer_count_pair*)c->table.p, t2_slots, d_pairs, pairs_capacity, c->d_status, st, mark_cb, &ma, spec, canon);
         c->launches += 4;
         c->p_recountable = true;
+        c->p_canonical = canon;
         c->p_seq = d_seq; c->p_off = d_row_off; c->p_pairs = d_pairs; c->p_pairs_cap = pairs_capacity;
         c->p_spectrum = spec != nullptr;
         if (spec) {
@@ -599,10 +603,10 @@ static int dev_count_impl(kmer_cuda_ctx* c, const char* d_seq, uint64_t n_bases,
         rc = ws(c, c->table, nbins * 8);
         if (rc) return rc;
         if (spec) {
-            launch_dense_table(c->di, a, (unsigned long long*)c->table.p, st);
+            launch_dense_table(c->di, a, (unsigned long long*)c->table.p, st, canon);
             launch_dense_spectrum(c->di, (const unsigned long long*)c->table.p, k, 0, 1, *spec, c->d_status, st);
         } else
-            launch_count_dense(c->di, a, (unsigned long long*)c->table.p, d_pairs, pairs_capacity, st);
+            launch_count_dense(c->di, a, (unsigned long long*)c->table.p, d_pairs, pairs_capacity, st, canon);
         c->launches += 2;
         mark(c, st, spec ? "count_dense+spectrum" : "count_dense+compact");
     } else if (algo == 2) {
@@ -613,7 +617,7 @@ static int dev_count_impl(kmer_cuda_ctx* c, const char* d_seq, uint64_t n_bases,
         if (rc) return rc;
         launch_hash_clear((kmer_count_pair*)c->table.p, n_slots, st);
         mark(c, st, "hash_clear");
-        launch_count_hash_insert(c->di, a, (kmer_count_pair*)c->table.p, n_slots, st);
+        launch_count_hash_insert(c->di, a, (kmer_count_pair*)c->table.p, n_slots, st, canon);
         mark(c, st, "count_hash_insert");
         if (spec) launch_hash_spectrum(c->di, (const kmer_count_pair*)c->table.p, n_slots, k, *spec, c->d_status, st);
         else launch_hash_compact(c->di, (const kmer_count_pair*)c->table.p, n_slots, k, d_pairs, pairs_capacity, c->d_status, st);
@@ -655,6 +659,25 @@ extern "C" int kmer_cuda_dev_count_spectrum(kmer_cuda_ctx* c, const char* d_seq,
     if (rc) return rc;
     const SpecOut o = spec_out(d_hist, hist_len, d_tail, tail_capacity);
     return dev_count_impl(c, d_seq, n_bases, d_row_off, n_rows, k, nullptr, 0, nullptr, 0, algo, stream, &o);
+}
+
+// canonical counting: the strand-specific entry points' contracts with min(code, reverse complement) as the group key
+extern "C" int kmer_cuda_dev_count_canonical(kmer_cuda_ctx* c, const char* d_seq, uint64_t n_bases, const uint64_t* d_row_off,
+                                             uint64_t n_rows, int k, uint64_t* d_uniq, uint64_t uniq_capacity, kmer_count_pair* d_pairs,
+                                             uint64_t pairs_capacity, int algo, void* stream) {
+    if (c && !d_uniq && uniq_capacity) return bad_arg(c, "d_uniq");
+    return dev_count_impl(c, d_seq, n_bases, d_row_off, n_rows, k, d_pairs, pairs_capacity, d_uniq, d_uniq ? uniq_capacity : 0, algo,
+                          stream, nullptr, true);
+}
+
+extern "C" int kmer_cuda_dev_count_canonical_spectrum(kmer_cuda_ctx* c, const char* d_seq, uint64_t n_bases, const uint64_t* d_row_off,
+                                                      uint64_t n_rows, int k, uint64_t* d_hist, uint64_t hist_len, kmer_count_pair* d_tail,
+                                                      uint64_t tail_capacity, int algo, void* stream) {
+    if (!c) return KMER_ERR_BAD_ARGUMENT;
+    int rc = spectrum_args(c, d_hist, hist_len, d_tail, tail_capacity);
+    if (rc) return rc;
+    const SpecOut o = spec_out(d_hist, hist_len, d_tail, tail_capacity);
+    return dev_count_impl(c, d_seq, n_bases, d_row_off, n_rows, k, nullptr, 0, nullptr, 0, algo, stream, &o, true);
 }
 
 extern "C" int kmer_cuda_dev_pairs_spectrum(kmer_cuda_ctx* c, const kmer_count_pair* d_pairs, uint64_t n, uint64_t* d_hist,
@@ -821,7 +844,7 @@ extern "C" int kmer_cuda_dev_finish(kmer_cuda_ctx* c, void* stream, kmer_dev_res
             a.status = c->d_status;
             status_reset_kernel<<<1, 1, 0, st>>>(c->d_status);          // also rewinds the tail cursor of the spectrum format
             launch_hash_clear((kmer_count_pair*)c->table.p, n_slots, st);
-            launch_count_hash_insert(c->di, a, (kmer_count_pair*)c->table.p, n_slots, st);
+            launch_count_hash_insert(c->di, a, (kmer_count_pair*)c->table.p, n_slots, st, c->p_canonical);
             if (c->p_spectrum) {                                        // what the leaf and tier 2 binned so far is void as well
                 const SpecOut o = spec_out(c->p_hist, c->p_hist_len, c->p_tail, c->p_tail_cap);
                 rc = spectrum_begin(c, o, st);
@@ -1368,7 +1391,7 @@ static int download_spectrum(kmer_cuda_ctx* c, uint64_t hist_len, const kmer_dev
 // second copy stream (PCIe is the bound of this call: the kernels hide under the copies).  FMT_SPECTRUM (hist_len >= 2): the
 // groups are binned on the device and nothing streams back but the histogram and the tail, once everything is counted.
 static int submit_count_common(kmer_cuda_ctx* c, const char* seq, const uint64_t* row_off, uint64_t n_rows, int k, CountFormat fmt,
-                               CountOut* o, uint64_t hist_len = 0) {
+                               CountOut* o, uint64_t hist_len = 0, bool canon = false) {
     CU(cudaSetDevice(c->di.device), "cudaSetDevice");
     if (n_rows && !row_off) return bad_arg(c, "row_off");
     const uint64_t n_bases = n_rows ? row_off[n_rows] : 0;
@@ -1400,14 +1423,12 @@ static int submit_count_common(kmer_cuda_ctx* c, const char* seq, const uint64_t
         if (!rc && n_rows) rc = h2d(c, c->off.p, row_off, (n_rows + 1) * 8, c->stream);
         if (rc) return rc;
         if (spectrum)
-            rc = kmer_cuda_dev_count_spectrum(c, (const char*)c->seq.p, n_bases, (const uint64_t*)c->off.p, n_rows, k, (uint64_t*)c->hist.p,
-                                              hist_len, (kmer_count_pair*)c->pairs.p, tail_cap, 0, KMER_OWN_STREAM);
-        else if (fmt == FMT_PAIRS)
-            rc = kmer_cuda_dev_count(c, (const char*)c->seq.p, n_bases, (const uint64_t*)c->off.p, n_rows, k, (kmer_count_pair*)c->pairs.p, cap,
-                                     0, KMER_OWN_STREAM);
+            rc = dev_count_impl(c, (const char*)c->seq.p, n_bases, (const uint64_t*)c->off.p, n_rows, k, nullptr, 0, nullptr, 0, 0,
+                                KMER_OWN_STREAM, &so, canon);
         else
-            rc = kmer_cuda_dev_count_split(c, (const char*)c->seq.p, n_bases, (const uint64_t*)c->off.p, n_rows, k, (uint64_t*)c->codes.p, cap,
-                                           (kmer_count_pair*)c->pairs.p, cap, KMER_OWN_STREAM);
+            rc = dev_count_impl(c, (const char*)c->seq.p, n_bases, (const uint64_t*)c->off.p, n_rows, k, (kmer_count_pair*)c->pairs.p, cap,
+                                fmt == FMT_PAIRS ? nullptr : (uint64_t*)c->codes.p, fmt == FMT_PAIRS ? 0 : cap, 0, KMER_OWN_STREAM,
+                                nullptr, canon);
         if (rc) return rc;
         rc = kmer_cuda_dev_finish(c, KMER_OWN_STREAM, &res);
         if (rc) return rc;
@@ -1452,7 +1473,7 @@ static int submit_count_common(kmer_cuda_ctx* c, const char* seq, const uint64_t
     ScanArgs a;
     rc = prepare_rows(c, d_off, n_bases, n_rows, k, st, &a, d_seq);
     if (rc) return rc;
-    PartitionPlan plan = make_partition_plan(c->p_expected_kmers, k);
+    PartitionPlan plan = make_partition_plan(c->p_expected_kmers, k, canon);
     rc = ws(c, c->fill, (size_t)plan.n_buckets * 8);
     if (!rc) rc = ws(c, c->recs, partition_record_bytes(plan));
     if (!rc) rc = ws(c, c->spill, partition_spill_bytes(plan));
@@ -1473,7 +1494,7 @@ static int submit_count_common(kmer_cuda_ctx* c, const char* seq, const uint64_t
         CU(cudaStreamWaitEvent(st, c->ev_in[i], 0), "wait");
         a.tile_begin = t0;
         a.tile_end = t1;
-        launch_partition(c->di, a, plan, (unsigned long long*)c->fill.p, c->recs.p, c->spill.p, st, false);
+        launch_partition(c->di, a, plan, (unsigned long long*)c->fill.p, c->recs.p, c->spill.p, st, false, canon);
         c->launches++;
     }
     mark(c, st, "minimizer_partition");
@@ -1484,7 +1505,7 @@ static int submit_count_common(kmer_cuda_ctx* c, const char* seq, const uint64_t
     for (int g = 0; g < n_groups; g++) {
         const uint32_t g0 = (uint32_t)((uint64_t)plan.n_buckets * g / n_groups), g1 = (uint32_t)((uint64_t)plan.n_buckets * (g + 1) / n_groups);
         launch_bucket_count(c->di, plan, k, (const unsigned long long*)c->fill.p, c->recs.p, c->spill.p, (uint32_t*)c->failed.p, d_pairs,
-                            cap, d_uniq, d_uniq ? cap : 0, c->d_status, st, g0, g1, spec);
+                            cap, d_uniq, d_uniq ? cap : 0, c->d_status, st, g0, g1, spec, canon);
         c->launches++;
         if (spectrum) break;
         CU(cudaMemcpyAsync(&c->h_ring[g], c->d_status, sizeof(DevStatus), cudaMemcpyDeviceToHost, st), "D2H status");
@@ -1493,13 +1514,14 @@ static int submit_count_common(kmer_cuda_ctx* c, const char* seq, const uint64_t
     mark(c, st, "bucket_count");
     MarkArg ma{c, st};
     launch_partition_tier2(c->di, plan, k, (const unsigned long long*)c->fill.p, c->recs.p, c->spill.p, (const uint32_t*)c->failed.p,
-                           (kmer_count_pair*)c->table.p, t2_slots, d_pairs, cap, c->d_status, st, mark_cb, &ma, spec);
+                           (kmer_count_pair*)c->table.p, t2_slots, d_pairs, cap, c->d_status, st, mark_cb, &ma, spec, canon);
     resolve_bad_row_kernel<<<1, 1, 0, st>>>(c->d_status, d_off, n_rows);
     c->launches += 5;
     CU(cudaGetLastError(), "count launch");
     c->p_recountable = true;
     c->p_seq = d_seq; c->p_off = d_off; c->p_pairs = d_pairs; c->p_pairs_cap = cap;
     c->p_spectrum = spectrum;
+    c->p_canonical = canon;
     if (spectrum) {
         c->p_hist = (uint64_t*)c->hist.p; c->p_hist_len = hist_len; c->p_tail = d_pairs; c->p_tail_cap = tail_cap;
         rc = kmer_cuda_dev_finish(c, KMER_OWN_STREAM, &res);      // input errors, tier 2, or a tier-3 recount
@@ -1626,6 +1648,44 @@ extern "C" int kmer_cuda_submit_count_spectrum(kmer_cuda_ctx* c, const char* seq
     if (n_kmers) *n_kmers = 0;
     CountOut o;
     int rc = submit_count_common(c, seq, row_off, n_rows, k, FMT_SPECTRUM, &o, hist_len);
+    if (rc) return rc;
+    *hist = o.hist;
+    *tail = o.pairs;
+    *n_tail = o.n_pairs;
+    if (n_kmers) *n_kmers = o.n_kmers;
+    return KMER_OK;
+}
+
+extern "C" int kmer_cuda_submit_count_canonical(kmer_cuda_ctx* c, const char* seq, const uint64_t* row_off, uint64_t n_rows, int k,
+                                                uint64_t** uniq_codes, uint64_t* n_unique, kmer_count_pair** pairs, uint64_t* n_pairs,
+                                                uint64_t* n_kmers) {
+    if (!c || !pairs || !n_pairs || (uniq_codes && !n_unique)) return KMER_ERR_BAD_ARGUMENT;
+    if (uniq_codes) { *uniq_codes = nullptr; *n_unique = 0; }
+    *pairs = nullptr;
+    *n_pairs = 0;
+    if (n_kmers) *n_kmers = 0;
+    CountOut o;
+    int rc = submit_count_common(c, seq, row_off, n_rows, k, uniq_codes ? FMT_SPLIT : FMT_PAIRS, &o, 0, true);
+    if (rc) return rc;
+    if (uniq_codes) {
+        *uniq_codes = (uint64_t*)o.uniq;
+        *n_unique = o.n_unique;
+    }
+    *pairs = o.pairs;
+    *n_pairs = o.n_pairs;
+    if (n_kmers) *n_kmers = o.n_kmers;
+    return KMER_OK;
+}
+
+extern "C" int kmer_cuda_submit_count_canonical_spectrum(kmer_cuda_ctx* c, const char* seq, const uint64_t* row_off, uint64_t n_rows,
+                                                         int k, uint64_t hist_len, uint64_t** hist, kmer_count_pair** tail,
+                                                         uint64_t* n_tail, uint64_t* n_kmers) {
+    if (!c || !hist || !tail || !n_tail || hist_len < 2) return KMER_ERR_BAD_ARGUMENT;
+    *hist = nullptr; *tail = nullptr;
+    *n_tail = 0;
+    if (n_kmers) *n_kmers = 0;
+    CountOut o;
+    int rc = submit_count_common(c, seq, row_off, n_rows, k, FMT_SPECTRUM, &o, hist_len, true);
     if (rc) return rc;
     *hist = o.hist;
     *tail = o.pairs;

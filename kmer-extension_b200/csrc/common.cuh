@@ -78,6 +78,50 @@ __device__ __forceinline__ uint32_t bits32(const uint32_t* bits, int b) {
 }
 
 // ---------------------------------------------------------------------------------------------
+// reverse complement (canonical counting: a k-mer and its reverse complement are one group).  Codes a=0 c=1 g=2 t=3 complement
+// to 3 - b = ~b, so rc is the bit-reversed complement with every 2-bit base put back in order.
+__host__ __device__ __forceinline__ uint64_t brev64(uint64_t x) {
+#ifdef __CUDA_ARCH__
+    return __brevll(x);
+#else
+    x = ((x >> 1) & 0x5555555555555555ull) | ((x & 0x5555555555555555ull) << 1);
+    x = ((x >> 2) & 0x3333333333333333ull) | ((x & 0x3333333333333333ull) << 2);
+    x = ((x >> 4) & 0x0F0F0F0F0F0F0F0Full) | ((x & 0x0F0F0F0F0F0F0F0Full) << 4);
+    x = ((x >> 8) & 0x00FF00FF00FF00FFull) | ((x & 0x00FF00FF00FF00FFull) << 8);
+    x = ((x >> 16) & 0x0000FFFF0000FFFFull) | ((x & 0x0000FFFF0000FFFFull) << 16);
+    return (x >> 32) | (x << 32);
+#endif
+}
+__host__ __device__ __forceinline__ uint32_t brev32(uint32_t x) {
+#ifdef __CUDA_ARCH__
+    return __brev(x);
+#else
+    return (uint32_t)(brev64(x) >> 32);
+#endif
+}
+// k-mer code (first base in the high bits of the low 2k) -> code of its reverse complement
+__host__ __device__ __forceinline__ uint64_t revcomp_code(uint64_t x, int k) {
+    uint64_t r = brev64(~x);
+    r = ((r >> 1) & 0x5555555555555555ull) | ((r & 0x5555555555555555ull) << 1);
+    return r >> (64 - 2 * k);
+}
+// the smaller of the two codes: also the smaller of the two lower-case texts (code order is memcmp order)
+__host__ __device__ __forceinline__ uint64_t canon_code(uint64_t x, int k) {
+    const uint64_t r = revcomp_code(x, k);
+    return r < x ? r : x;
+}
+// the same for the top-aligned m-mer that mmer_hash takes (its 2m top bits; the bits below are zero in the result)
+__host__ __device__ __forceinline__ uint32_t revcomp_mmer(uint32_t top, int m) {
+    uint32_t r = brev32(~top);
+    r = ((r >> 1) & 0x55555555u) | ((r & 0x55555555u) << 1);
+    return r << (32 - 2 * m);
+}
+__host__ __device__ __forceinline__ uint32_t canon_mmer(uint32_t top, uint32_t himask, int m) {
+    const uint32_t f = top & himask, r = revcomp_mmer(top, m);
+    return r < f ? r : f;
+}
+
+// ---------------------------------------------------------------------------------------------
 // hashes
 __device__ __host__ __forceinline__ uint64_t mix64(uint64_t x) {   // murmur3 finaliser (bijective)
     x ^= x >> 33; x *= 0xff51afd7ed558ccdull;

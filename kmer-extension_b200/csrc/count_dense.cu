@@ -7,6 +7,7 @@ namespace kmer {
 
 constexpr int kSmemDenseMaxK = 6;  // 4096 bins * 4 B = 16 KB
 
+template <bool CANON = false>
 __global__ void __launch_bounds__(NT) count_dense_smem_kernel(ScanArgs a, unsigned long long* __restrict__ table) {
     __shared__ ScanSmem s;
     __shared__ uint32_t bins[1 << (2 * kSmemDenseMaxK)];
@@ -17,7 +18,7 @@ __global__ void __launch_bounds__(NT) count_dense_smem_kernel(ScanArgs a, unsign
 #pragma unroll 4
         for (int j = 0; j < TILE / NT; j++) {
             int i = j * NT + threadIdx.x;
-            if (sc.valid(i)) atomicAdd(&bins[(uint32_t)sc.code(i)], 1u);
+            if (sc.valid(i)) atomicAdd(&bins[(uint32_t)(CANON ? canon_code(sc.code(i), a.k) : sc.code(i))], 1u);
         }
         sc.release();
     }
@@ -28,6 +29,7 @@ __global__ void __launch_bounds__(NT) count_dense_smem_kernel(ScanArgs a, unsign
     }
 }
 
+template <bool CANON = false>
 __global__ void __launch_bounds__(NT) count_dense_global_kernel(ScanArgs a, unsigned long long* __restrict__ table) {
     __shared__ ScanSmem s;
     TileScanner sc(a, s);
@@ -35,7 +37,7 @@ __global__ void __launch_bounds__(NT) count_dense_global_kernel(ScanArgs a, unsi
 #pragma unroll 4
         for (int j = 0; j < TILE / NT; j++) {
             int i = j * NT + threadIdx.x;
-            if (sc.valid(i)) atomicAdd(&table[sc.code(i)], 1ull);
+            if (sc.valid(i)) atomicAdd(&table[CANON ? canon_code(sc.code(i), a.k) : sc.code(i)], 1ull);
         }
         sc.release();
     }
@@ -67,15 +69,20 @@ __global__ void dense_compact_kernel(const unsigned long long* __restrict__ tabl
     if (lane == 0 && total) atomicAdd(&status->n_kmers, total);
 }
 
-void launch_dense_table(const DeviceInfo& di, const ScanArgs& a, unsigned long long* d_table, cudaStream_t st) {
+void launch_dense_table(const DeviceInfo& di, const ScanArgs& a, unsigned long long* d_table, cudaStream_t st, bool canon) {
     uint64_t nbins = 1ull << (2 * a.k);
     cudaMemsetAsync(d_table, 0, nbins * sizeof(unsigned long long), st);
     uint64_t n_tiles = (a.n_bases + TILE - 1) / TILE;
     if (n_tiles) {
         uint64_t grid = (uint64_t)di.sm_count * 6;
         if (grid > n_tiles) grid = n_tiles;
-        if (a.k <= kSmemDenseMaxK) count_dense_smem_kernel<<<(unsigned)grid, NT, 0, st>>>(a, d_table);
-        else count_dense_global_kernel<<<(unsigned)grid, NT, 0, st>>>(a, d_table);
+        if (a.k <= kSmemDenseMaxK) {
+            if (canon) count_dense_smem_kernel<true><<<(unsigned)grid, NT, 0, st>>>(a, d_table);
+            else count_dense_smem_kernel<<<(unsigned)grid, NT, 0, st>>>(a, d_table);
+        } else {
+            if (canon) count_dense_global_kernel<true><<<(unsigned)grid, NT, 0, st>>>(a, d_table);
+            else count_dense_global_kernel<<<(unsigned)grid, NT, 0, st>>>(a, d_table);
+        }
     }
 }
 
@@ -89,8 +96,8 @@ void launch_dense_emit(const DeviceInfo& di, const unsigned long long* d_table, 
 }
 
 void launch_count_dense(const DeviceInfo& di, const ScanArgs& a, unsigned long long* d_table, kmer_count_pair* d_pairs,
-                        uint64_t capacity, cudaStream_t st) {
-    launch_dense_table(di, a, d_table, st);
+                        uint64_t capacity, cudaStream_t st, bool canon) {
+    launch_dense_table(di, a, d_table, st, canon);
     launch_dense_emit(di, d_table, a.k, 0, 1, d_pairs, capacity, a.status, st);
 }
 

@@ -20,6 +20,7 @@ __device__ __forceinline__ void table_add(kmer_count_pair* slots, uint64_t mask,
     }
 }
 
+template <bool CANON = false>
 __global__ void __launch_bounds__(NT) count_hash_insert_kernel(ScanArgs a, kmer_count_pair* __restrict__ slots, uint64_t mask) {
     __shared__ ScanSmem s;
     TileScanner sc(a, s);
@@ -30,6 +31,7 @@ __global__ void __launch_bounds__(NT) count_hash_insert_kernel(ScanArgs a, kmer_
             int i = j * NT + threadIdx.x;
             bool v = sc.valid(i);
             uint64_t code = sc.code(i);
+            if (CANON) code = canon_code(code, a.k);       // never kEmpty: canon('t'*32) = 'a'*32
             // warp-aggregate equal keys (repetitive sequence => many equal neighbours)
             uint32_t vm = __ballot_sync(0xffffffffu, v);
             uint32_t same = __match_any_sync(0xffffffffu, code) & vm;
@@ -83,12 +85,13 @@ void launch_hash_clear(kmer_count_pair* d_slots, uint64_t n_slots, cudaStream_t 
 }
 
 void launch_count_hash_insert(const DeviceInfo& di, const ScanArgs& a, kmer_count_pair* d_slots, uint64_t n_slots,
-                              cudaStream_t st) {
+                              cudaStream_t st, bool canon) {
     uint64_t n_tiles = (a.n_bases + TILE - 1) / TILE;
     if (!n_tiles) return;
     uint64_t grid = (uint64_t)di.sm_count * 6;
     if (grid > n_tiles) grid = n_tiles;
-    count_hash_insert_kernel<<<(unsigned)grid, NT, 0, st>>>(a, d_slots, n_slots - 1);
+    if (canon) count_hash_insert_kernel<true><<<(unsigned)grid, NT, 0, st>>>(a, d_slots, n_slots - 1);
+    else count_hash_insert_kernel<<<(unsigned)grid, NT, 0, st>>>(a, d_slots, n_slots - 1);
 }
 
 // gated != 0: the table is tier 2's and is only looked at if the device decided to run tier 2 (DevStatus::t2_mode == 1);

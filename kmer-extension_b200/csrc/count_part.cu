@@ -62,7 +62,11 @@ struct alignas(16) Rec<2> {
 #ifndef PART_MINB
 #define PART_MINB 3
 #endif
-template <int W, int RECW>
+// CANON: canonical counting needs a k-mer and its reverse complement in one bucket, so the minimizer is strand-symmetric: the
+// hashed m-mer is the canonical one (min(m-mer, rc)), and the W m-mers of a window sit symmetrically in it, offset by
+// (k - m - W + 1) / 2 bases (make_partition_plan keeps that even).  Then a k-mer and its reverse complement hash the same set of
+// canonical m-mers.  The records still carry the forward bases.
+template <int W, int RECW, bool CANON = false>
 __global__ void __launch_bounds__(NT, PART_MINB) partition_kernel(ScanArgs a, PartitionPlan plan, unsigned long long* __restrict__ fill,
                                                        Rec<RECW>* __restrict__ recs, Rec<RECW>* __restrict__ spill) {
     __shared__ ScanSmem s;
@@ -119,7 +123,15 @@ __global__ void __launch_bounds__(NT, PART_MINB) partition_kernel(ScanArgs a, Pa
         // window 16t-1 (the previous thread's last) is looked at as well, so that runs continue across threads
         uint32_t w[3];
         w[0] = s.packed[t]; w[1] = s.packed[t + 1]; w[2] = s.packed[t + 2];
-        const uint32_t wm1 = t ? s.packed[t - 1] : 0u;
+        uint32_t wm1 = t ? s.packed[t - 1] : 0u;
+        if (CANON) {                                                  // the m-mers of window j start at base j + off
+            const int sh = k - m - W + 1;                             // 2 * off: off <= 5, so j + off <= 31 below
+            const uint32_t w3 = s.packed[t + 3];
+            wm1 = __funnelshift_l(w[0], wm1, sh);
+            w[0] = __funnelshift_l(w[1], w[0], sh);
+            w[1] = __funnelshift_l(w[2], w[1], sh);
+            w[2] = __funnelshift_l(w3, w[2], sh);
+        }
         // validity of the windows: no row start in (i, i+k-1], and inside the input
         uint32_t vmask = 0;      // bit j+1: window j is valid (j = -1 .. 15)
         {
@@ -149,7 +161,7 @@ __global__ void __launch_bounds__(NT, PART_MINB) partition_kernel(ScanArgs a, Pa
                     const int q = j >> 4, sh = (j & 15) * 2;
                     top = __funnelshift_l(w[q + 1], w[q], sh);
                 }
-                h[j + 1] = mmer_hash(top, himask, m);
+                h[j + 1] = mmer_hash(CANON ? canon_mmer(top, himask, m) : top, himask, m);
             }
             // sliding minimum over W consecutive m-mers: log-steps up to the largest power of two P <= W, then two
             // overlapping P-windows cover a W-window
@@ -396,7 +408,7 @@ __device__ __forceinline__ BucketInfo bucket_info(const unsigned long long* __re
     return bi;
 }
 
-template <int RECW, bool SPLIT, bool SPEC = false>
+template <int RECW, bool SPLIT, bool SPEC = false, bool CANON = false>
 __global__ void __launch_bounds__(LEAF_THREADS, LEAF_MINB) bucket_count_kernel(PartitionPlan plan, int k,
                                                                        const unsigned long long* __restrict__ fill,
                                                                        const Rec<RECW>* __restrict__ recs,
@@ -495,6 +507,8 @@ __global__ void __launch_bounds__(LEAF_THREADS, LEAF_MINB) bucket_count_kernel(P
             lds128(rec_s + 16 * r, hi, lo);
             return (j ? ((hi << (2 * j)) | (lo >> (64 - 2 * j))) : hi) >> kshift;
         };
+        // CANON: every key is the canonical code of its window, formed where mark and count read it.  A record may then hold
+        // both x and rc(x): nothing below assumes the keys of a record are distinct.
         // ---- index: thread t numbers the k-mers of records [t*c, t*c + c)
         const uint32_t nrec = cur.nrec;
         {
@@ -536,6 +550,7 @@ __global__ void __launch_bounds__(LEAF_THREADS, LEAF_MINB) bucket_count_kernel(P
             const uint32_t j = (uint32_t)(t + i * LEAF_THREADS) - lds16(p_s + 2 * r);
             if (j < rec_len(r)) {                                       // not in the padding behind the warp's last record
                 key[i] = window(r, j);
+                if (CANON) key[i] = canon_code(key[i], k);
                 if (RECW == 2 && key[i] == kEmpty) special++;           // k == 32, 't'*32: kept out of the tables
                 else {
                     valid |= 1u << i;
@@ -603,6 +618,7 @@ __global__ void __launch_bounds__(LEAF_THREADS, LEAF_MINB) bucket_count_kernel(P
                         const uint32_t ki = lds16(slow_s + 2 * idx), blk = ki >> 5;
                         const uint32_t r = lds32(blk_s + 4 * blk) + __popc(lds32(mask_s + 4 * blk) & ((2u << (ki & 31u)) - 2u));
                         skey = window(r, ki - lds16(p_s + 2 * r));
+                        if (CANON) skey = canon_code(skey, k);
                         x = leaf_mix(skey) * 0x2C1B3C6Du;               // decorrelate from the cell index
                         tries = 0;
                         active = true;
@@ -968,7 +984,7 @@ __device__ __forceinline__ void global_table_add(kmer_count_pair* slots, uint64_
     }
 }
 
-template <int RECW>
+template <int RECW, bool CANON>
 __device__ __forceinline__ void tier2_add_record(const Rec<RECW>* p, int kshift, kmer_count_pair* slots, uint64_t mask,
                                                  DevStatus* status, bool active) {
     uint64_t hi = 0, lo = 0;
@@ -984,6 +1000,7 @@ __device__ __forceinline__ void tier2_add_record(const Rec<RECW>* p, int kshift,
         bool v = o < L;
         uint64_t win = (RECW == 1 || o == 0) ? (hi << (2 * o)) : ((hi << (2 * o)) | (lo >> (64 - 2 * o)));
         uint64_t key = win >> kshift;
+        if (CANON) key = canon_code(key, (64 - kshift) >> 1);   // the leaf's one-k-mer spill records are canonical already
         uint32_t vm = __ballot_sync(0xffffffffu, v);
         uint32_t same = __match_any_sync(0xffffffffu, key) & vm;     // repetitive input: aggregate equal keys
         if (v && lane == __ffs(same) - 1) {
@@ -1017,7 +1034,7 @@ __global__ void __launch_bounds__(256) tier2_clear_kernel(uint4* __restrict__ sl
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_slots; i += stride) slots[i] = make_uint4(~0u, ~0u, ~0u, ~0u);
 }
 
-template <int RECW>
+template <int RECW, bool CANON = false>
 __global__ void __launch_bounds__(256) tier2_insert_kernel(PartitionPlan plan, int k, const unsigned long long* __restrict__ fill,
                                                            const Rec<RECW>* __restrict__ recs, const uint32_t* __restrict__ failed_ids,
                                                            const Rec<RECW>* __restrict__ spill, kmer_count_pair* __restrict__ slots,
@@ -1032,14 +1049,14 @@ __global__ void __launch_bounds__(256) tier2_insert_kernel(PartitionPlan plan, i
         const Rec<RECW>* base = recs + (uint64_t)b * plan.cap;
         for (uint32_t r0 = 0; r0 < nrec; r0 += blockDim.x) {
             uint32_t r = r0 + threadIdx.x;
-            tier2_add_record<RECW>(base + min(r, nrec - 1), kshift, slots, mask, status, r < nrec);
+            tier2_add_record<RECW, CANON>(base + min(r, nrec - 1), kshift, slots, mask, status, r < nrec);
         }
     }
     const uint64_t n_spill = min((uint64_t)status->n_spill, (uint64_t)plan.spill_cap);
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
     for (uint64_t r0 = (uint64_t)blockIdx.x * blockDim.x; r0 < n_spill; r0 += stride) {
         uint64_t r = r0 + threadIdx.x;
-        tier2_add_record<RECW>(spill + min(r, n_spill - 1), kshift, slots, mask, status, r < n_spill);
+        tier2_add_record<RECW, CANON>(spill + min(r, n_spill - 1), kshift, slots, mask, status, r < n_spill);
     }
 }
 
@@ -1178,7 +1195,16 @@ void launch_scatter_refine(const DeviceInfo& di, const ScanArgs& a, const Partit
 static int g_forced_window = 0;
 void partition_force_window(int w) { g_forced_window = w; }
 
-PartitionPlan make_partition_plan(uint64_t n_kmers, int k) {
+// m-mer length for window w: k - w + 1, capped at 16 bases.  Canonical counting (partition_kernel<.., true>) centres the w m-mers
+// in the k-mer, which needs k - w + 1 - m even, and has only about 4^m / 2 distinct (canonical) m-mers.
+static int plan_m(int k, int w, bool canon) {
+    int m = k - w + 1 > 16 ? 16 : k - w + 1;
+    if (canon && ((k - w + 1 - m) & 1)) m--;
+    return m;
+}
+static bool mmers_fine_enough(int m, bool canon, uint64_t nb) { return ldexp(1.0, 2 * m - (canon ? 1 : 0)) >= 30.0 * (double)nb; }
+
+PartitionPlan make_partition_plan(uint64_t n_kmers, int k, bool canon) {
     PartitionPlan p{};
     // minimizer window: w windows share a record while their minimizer (an m-mer, m = k - w + 1, capped at 16 bases) stays the same
     const uint32_t target = TARGET_KMERS_PER_BUCKET;
@@ -1197,9 +1223,9 @@ PartitionPlan make_partition_plan(uint64_t n_kmers, int k) {
         p.w = ws[3];
         p.even = 1;                                        // nothing fits: the narrowest window, m-mers spread by a second hash
         for (int i = 0; i < 4; i++) {
-            const int m = k - ws[i] + 1 > 16 ? 16 : k - ws[i] + 1;
+            const int m = plan_m(k, ws[i], canon);
             if (ws[i] == 9 && k > 22) continue;            // 9 windows do not fit an 8-byte record (30 bases) beyond k = 22
-            if (ldexp(1.0, 2 * m) >= 30.0 * (double)nb) { p.w = ws[i]; p.even = 0; break; }
+            if (mmers_fine_enough(m, canon, nb)) { p.w = ws[i]; p.even = 0; break; }
         }
     }
     if (g_forced_window) {                                 // tests only (kmer_cuda_test_force_window): must suit the record width and k
@@ -1207,12 +1233,10 @@ PartitionPlan make_partition_plan(uint64_t n_kmers, int k) {
         const bool ok = p.recw == 1 ? (w == 4 || w == 6 || w == 8 || w == 9) : (w == 8 || w == 12 || w == 16);
         if (ok && k - w + 1 >= 2) {
             p.w = w;
-            const int mf = k - w + 1 > 16 ? 16 : k - w + 1;
-            p.even = ldexp(1.0, 2 * mf) >= 30.0 * (double)nb ? 0 : 1;
+            p.even = mmers_fine_enough(plan_m(k, w, canon), canon, nb) ? 0 : 1;
         }
     }
-    int m = k - p.w + 1;
-    p.m = m > 16 ? 16 : m;
+    p.m = plan_m(k, p.w, canon);
     p.rmax = p.recw == 1 ? (30 - k + 1 > 16 ? 16 : 30 - k + 1) : 16;
     p.n_buckets = (uint32_t)nb;
     p.hash_buckets = p.n_buckets;
@@ -1231,19 +1255,30 @@ size_t partition_record_bytes(const PartitionPlan& p) { return (size_t)p.n_bucke
 size_t partition_spill_bytes(const PartitionPlan& p) { return (size_t)p.spill_cap * (p.recw == 1 ? 8 : 16); }
 
 void launch_partition(const DeviceInfo& di, const ScanArgs& a, const PartitionPlan& p, unsigned long long* d_fill,
-                      void* d_recs, void* d_spill, cudaStream_t st, bool clear_fill) {
+                      void* d_recs, void* d_spill, cudaStream_t st, bool clear_fill, bool canon) {
     if (clear_fill) cudaMemsetAsync(d_fill, 0, (size_t)p.n_buckets * sizeof(unsigned long long), st);
     uint64_t n_tiles = a.tile_end ? a.tile_end - a.tile_begin : (a.n_bases + TILE - 1) / TILE;
     uint64_t grid = (uint64_t)di.sm_count * PART_MINB;
     if (grid > n_tiles) grid = n_tiles;
     if (!n_tiles) return;
-    if (p.w == 4) partition_kernel<4, 1><<<(unsigned)grid, NT, 0, st>>>(a, p, d_fill, (Rec<1>*)d_recs, (Rec<1>*)d_spill);
-    else if (p.w == 6) partition_kernel<6, 1><<<(unsigned)grid, NT, 0, st>>>(a, p, d_fill, (Rec<1>*)d_recs, (Rec<1>*)d_spill);
-    else if (p.w == 9) partition_kernel<9, 1><<<(unsigned)grid, NT, 0, st>>>(a, p, d_fill, (Rec<1>*)d_recs, (Rec<1>*)d_spill);
-    else if (p.w == 12) partition_kernel<12, 2><<<(unsigned)grid, NT, 0, st>>>(a, p, d_fill, (Rec<2>*)d_recs, (Rec<2>*)d_spill);
-    else if (p.w == 8 && p.recw == 1) partition_kernel<8, 1><<<(unsigned)grid, NT, 0, st>>>(a, p, d_fill, (Rec<1>*)d_recs, (Rec<1>*)d_spill);
-    else if (p.w == 8) partition_kernel<8, 2><<<(unsigned)grid, NT, 0, st>>>(a, p, d_fill, (Rec<2>*)d_recs, (Rec<2>*)d_spill);
-    else partition_kernel<16, 2><<<(unsigned)grid, NT, 0, st>>>(a, p, d_fill, (Rec<2>*)d_recs, (Rec<2>*)d_spill);
+#define KMER_PART(W_, R_) partition_kernel<W_, R_, C_><<<(unsigned)grid, NT, 0, st>>>(a, p, d_fill, (Rec<R_>*)d_recs, (Rec<R_>*)d_spill)
+#define KMER_PART_ALL                                                                 \
+    if (p.w == 4) KMER_PART(4, 1);                                                    \
+    else if (p.w == 6) KMER_PART(6, 1);                                               \
+    else if (p.w == 9) KMER_PART(9, 1);                                               \
+    else if (p.w == 12) KMER_PART(12, 2);                                             \
+    else if (p.w == 8 && p.recw == 1) KMER_PART(8, 1);                                \
+    else if (p.w == 8) KMER_PART(8, 2);                                               \
+    else KMER_PART(16, 2)
+    if (canon) {
+        constexpr bool C_ = true;
+        KMER_PART_ALL;
+    } else {
+        constexpr bool C_ = false;
+        KMER_PART_ALL;
+    }
+#undef KMER_PART_ALL
+#undef KMER_PART
 }
 
 // p.n_buckets = buckets counted HERE (all of them on one GPU, the owned range when sharded)
@@ -1266,6 +1301,8 @@ static void leaf_configure(size_t smem) {
     cudaFuncSetAttribute(bucket_count_kernel<RW, __VA_ARGS__>, cudaFuncAttributePreferredSharedMemoryCarveout, 100)
     KMER_LEAF_CONF(1, false); KMER_LEAF_CONF(1, true); KMER_LEAF_CONF(2, false); KMER_LEAF_CONF(2, true);
     KMER_LEAF_CONF(1, false, true); KMER_LEAF_CONF(2, false, true);
+    KMER_LEAF_CONF(1, false, false, true); KMER_LEAF_CONF(1, true, false, true); KMER_LEAF_CONF(2, false, false, true);
+    KMER_LEAF_CONF(2, true, false, true); KMER_LEAF_CONF(1, false, true, true); KMER_LEAF_CONF(2, false, true, true);
 #undef KMER_LEAF_CONF
     configured[dev] = smem;
 }
@@ -1273,7 +1310,7 @@ static void leaf_configure(size_t smem) {
 void launch_bucket_count(const DeviceInfo& di, const PartitionPlan& p, int k, const unsigned long long* d_fill,
                          const void* d_recs, void* d_spill, uint32_t* d_failed_ids, kmer_count_pair* d_pairs, uint64_t capacity,
                          uint64_t* d_uniq, uint64_t uniq_capacity, DevStatus* d_status, cudaStream_t st, uint32_t bucket_begin,
-                         uint32_t bucket_end, const SpecOut* spec) {
+                         uint32_t bucket_end, const SpecOut* spec, bool canon) {
     if (bucket_end == 0 || bucket_end > p.n_buckets) bucket_end = p.n_buckets;
     if (bucket_begin >= bucket_end) return;
     const size_t leaf_smem = leaf_smem_bytes(p) + (spec ? SPEC_SBINS * 4 : 0);
@@ -1283,32 +1320,34 @@ void launch_bucket_count(const DeviceInfo& di, const PartitionPlan& p, int k, co
     uint64_t lgrid = (uint64_t)di.sm_count * per_sm;
     if (lgrid > bucket_end - bucket_begin) lgrid = bucket_end - bucket_begin;
     leaf_configure(leaf_smem_bytes(p));
-    if (spec) {
-#define KMER_LEAF_SPEC(RW)                                                                                                        \
-    bucket_count_kernel<RW, false, true><<<(unsigned)lgrid, LEAF_THREADS, leaf_smem, st>>>(                                        \
+#define KMER_LEAF_SPEC(RW, CN)                                                                                                    \
+    bucket_count_kernel<RW, false, true, CN><<<(unsigned)lgrid, LEAF_THREADS, leaf_smem, st>>>(                                    \
         p, k, d_fill, (const Rec<RW>*)d_recs, spec->tail, spec->tail_cap, reinterpret_cast<uint64_t*>(spec->hist), spec->hist_len, \
         d_failed_ids, (Rec<RW>*)d_spill, d_status, bucket_begin, bucket_end)
-        if (p.recw == 1) KMER_LEAF_SPEC(1);
-        else KMER_LEAF_SPEC(2);
-#undef KMER_LEAF_SPEC
-        return;
-    }
-#define KMER_LEAF_GO(RW, SP)                                                                                                            \
-    bucket_count_kernel<RW, SP><<<(unsigned)lgrid, LEAF_THREADS, leaf_smem, st>>>(p, k, d_fill, (const Rec<RW>*)d_recs, d_pairs, capacity, \
+#define KMER_LEAF_GO(RW, SP, CN)                                                                                                        \
+    bucket_count_kernel<RW, SP, false, CN><<<(unsigned)lgrid, LEAF_THREADS, leaf_smem, st>>>(p, k, d_fill, (const Rec<RW>*)d_recs, d_pairs, capacity, \
                                                                                   d_uniq, uniq_capacity, d_failed_ids, (Rec<RW>*)d_spill, d_status, bucket_begin, bucket_end)
-    if (p.recw == 1) { if (d_uniq) KMER_LEAF_GO(1, true); else KMER_LEAF_GO(1, false); }
-    else { if (d_uniq) KMER_LEAF_GO(2, true); else KMER_LEAF_GO(2, false); }
+#define KMER_LEAF_ALL(CN)                                                                                    \
+    if (spec) {                                                                                              \
+        if (p.recw == 1) KMER_LEAF_SPEC(1, CN);                                                              \
+        else KMER_LEAF_SPEC(2, CN);                                                                          \
+    } else if (p.recw == 1) { if (d_uniq) KMER_LEAF_GO(1, true, CN); else KMER_LEAF_GO(1, false, CN); }      \
+    else { if (d_uniq) KMER_LEAF_GO(2, true, CN); else KMER_LEAF_GO(2, false, CN); }
+    if (canon) { KMER_LEAF_ALL(true) }
+    else { KMER_LEAF_ALL(false) }
+#undef KMER_LEAF_ALL
 #undef KMER_LEAF_GO
+#undef KMER_LEAF_SPEC
 }
 
 void launch_count_partition(const DeviceInfo& di, const ScanArgs& a, const PartitionPlan& p, unsigned long long* d_fill,
                             void* d_recs, void* d_spill, uint32_t* d_failed_ids, kmer_count_pair* d_pairs, uint64_t capacity,
                             uint64_t* d_uniq, uint64_t uniq_capacity, cudaStream_t st, void (*mark)(void*, const char*), void* mark_arg,
-                            const SpecOut* spec) {
-    launch_partition(di, a, p, d_fill, d_recs, d_spill, st);
+                            const SpecOut* spec, bool canon) {
+    launch_partition(di, a, p, d_fill, d_recs, d_spill, st, true, canon);
     if (mark) mark(mark_arg, "minimizer_partition");
     launch_bucket_count(di, p, a.k, d_fill, d_recs, d_spill, d_failed_ids, d_pairs, capacity, d_uniq, uniq_capacity, a.status, st, 0, 0,
-                        spec);
+                        spec, canon);
     if (mark) mark(mark_arg, "bucket_count");
 }
 
@@ -1321,16 +1360,15 @@ uint64_t tier2_table_slots(uint64_t n_kmers) {
 void launch_partition_tier2(const DeviceInfo& di, const PartitionPlan& p, int k, const unsigned long long* d_fill,
                             const void* d_recs, const void* d_spill, const uint32_t* d_failed_ids, kmer_count_pair* d_slots,
                             uint64_t n_slots, kmer_count_pair* d_pairs, uint64_t capacity, DevStatus* d_status, cudaStream_t st,
-                            void (*mark)(void*, const char*), void* mark_arg, const SpecOut* spec) {
+                            void (*mark)(void*, const char*), void* mark_arg, const SpecOut* spec, bool canon) {
     const unsigned grid = (unsigned)di.sm_count * 8;
     tier2_decide_kernel<<<1, 1, 0, st>>>(p, n_slots, d_status);
     tier2_clear_kernel<<<grid, 256, 0, st>>>((uint4*)d_slots, d_status);
-    if (p.recw == 1)
-        tier2_insert_kernel<1><<<grid, 256, 0, st>>>(p, k, d_fill, (const Rec<1>*)d_recs, d_failed_ids, (const Rec<1>*)d_spill,
-                                                     d_slots, d_status);
-    else
-        tier2_insert_kernel<2><<<grid, 256, 0, st>>>(p, k, d_fill, (const Rec<2>*)d_recs, d_failed_ids, (const Rec<2>*)d_spill,
-                                                     d_slots, d_status);
+#define KMER_T2(R_, C_) tier2_insert_kernel<R_, C_><<<grid, 256, 0, st>>>(p, k, d_fill, (const Rec<R_>*)d_recs, d_failed_ids, \
+                                                                       (const Rec<R_>*)d_spill, d_slots, d_status)
+    if (p.recw == 1) { if (canon) KMER_T2(1, true); else KMER_T2(1, false); }
+    else { if (canon) KMER_T2(2, true); else KMER_T2(2, false); }
+#undef KMER_T2
     if (mark) mark(mark_arg, "tier2_insert");
     if (spec) launch_hash_spectrum(di, d_slots, n_slots, k, *spec, d_status, st, 1);   // + the k == 32 special key
     else launch_hash_compact(di, d_slots, n_slots, k, d_pairs, capacity, d_status, st, 1);

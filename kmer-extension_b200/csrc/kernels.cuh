@@ -37,10 +37,11 @@ void launch_extract(const DeviceInfo& di, const ScanArgs& a, const uint32_t* d_t
 
 // count_dense.cu --------------------------------------------------------------------------------
 // k <= 13: direct-addressed counters (4^k uint64, zeroed here), then compaction of non-zero bins
+// canon: canonical counting -- every window is binned under min(code, reverse complement)
 void launch_count_dense(const DeviceInfo& di, const ScanArgs& a, unsigned long long* d_table,
-                        kmer_count_pair* d_pairs, uint64_t capacity, cudaStream_t st);
+                        kmer_count_pair* d_pairs, uint64_t capacity, cudaStream_t st, bool canon = false);
 
-void launch_dense_table(const DeviceInfo& di, const ScanArgs& a, unsigned long long* d_table, cudaStream_t st);
+void launch_dense_table(const DeviceInfo& di, const ScanArgs& a, unsigned long long* d_table, cudaStream_t st, bool canon = false);
 void launch_dense_emit(const DeviceInfo& di, const unsigned long long* d_table, int k, uint32_t rank, uint32_t n_ranks,
                        kmer_count_pair* d_pairs, uint64_t capacity, DevStatus* d_status, cudaStream_t st);
 
@@ -48,7 +49,7 @@ void launch_dense_emit(const DeviceInfo& di, const unsigned long long* d_table, 
 // open-addressing table of (code,count) slots in HBM; slots must be filled with 0xFF bytes
 void launch_hash_clear(kmer_count_pair* d_slots, uint64_t n_slots, cudaStream_t st);
 void launch_count_hash_insert(const DeviceInfo& di, const ScanArgs& a, kmer_count_pair* d_slots, uint64_t n_slots,
-                              cudaStream_t st);
+                              cudaStream_t st, bool canon = false);
 void launch_merge_pairs(const DeviceInfo& di, const kmer_count_pair* d_in, uint64_t n, uint32_t rank, uint32_t n_ranks,
                         kmer_count_pair* d_slots, uint64_t n_slots, DevStatus* d_status, cudaStream_t st);
 // appends every occupied slot (+ the k==32 special key) to d_pairs, bumping status->n_distinct
@@ -78,7 +79,8 @@ struct PartitionPlan {
     int even;             // 1: spread the m-mers over the buckets by a second hash (fewer than 30 m-mers per bucket: the load-aware
                           // map of bucket_position() cannot split an m-mer); 0: buckets of equal expected load
 };
-PartitionPlan make_partition_plan(uint64_t n_kmers, int k);
+// canon: the plan of canonical counting (the strand-symmetric minimizer of partition_kernel<.., true>: m may be one base shorter)
+PartitionPlan make_partition_plan(uint64_t n_kmers, int k, bool canon = false);
 void partition_force_window(int w);   // tests: 0 = automatic
 // two write-combining passes (scatter.cuh): column -> n_coarse partitions (one segment per scatter CTA) -> fine buckets
 struct ScatterPlan {
@@ -105,15 +107,17 @@ size_t partition_spill_bytes(const PartitionPlan& p);
 void launch_count_partition(const DeviceInfo& di, const ScanArgs& a, const PartitionPlan& p, unsigned long long* d_fill,
                             void* d_recs, void* d_spill, uint32_t* d_failed_ids, kmer_count_pair* d_pairs, uint64_t capacity,
                             uint64_t* d_uniq, uint64_t uniq_capacity, cudaStream_t st, void (*mark)(void*, const char*), void* mark_arg,
-                            const SpecOut* spec = nullptr);
+                            const SpecOut* spec = nullptr, bool canon = false);
 // a.tile_begin/tile_end: the tiles this launch walks (a column that arrives in pieces); clear_fill = false appends to the regions
 void launch_partition(const DeviceInfo& di, const ScanArgs& a, const PartitionPlan& p, unsigned long long* d_fill,
-                      void* d_recs, void* d_spill, cudaStream_t st, bool clear_fill = true);
+                      void* d_recs, void* d_spill, cudaStream_t st, bool clear_fill = true, bool canon = false);
 void launch_bucket_count(const DeviceInfo& di, const PartitionPlan& p, int k, const unsigned long long* d_fill,
                          const void* d_recs, void* d_spill, uint32_t* d_failed_ids, kmer_count_pair* d_pairs, uint64_t capacity,
                          uint64_t* d_uniq, uint64_t uniq_capacity, DevStatus* d_status, cudaStream_t st, uint32_t bucket_begin = 0,
-                         uint32_t bucket_end = 0, const SpecOut* spec = nullptr);
+                         uint32_t bucket_end = 0, const SpecOut* spec = nullptr, bool canon = false);
 // bucket_begin/bucket_end: the buckets this launch counts (0, 0: all) -- results can leave while later buckets are counted.
+// canon: canonical counting (keys canonicalized where the leaf forms them; the plan must come from make_partition_plan(.., true)
+// and the records from launch_partition(.., canon = true)).
 // d_uniq != nullptr: split result format -- k-mers proven unique on chip are written as bare codes to d_uniq (counted in
 // DevStatus::n_unique), everything else as (k-mer, count) pairs.  spec != nullptr: the spectrum result format instead (d_pairs,
 // d_uniq unused): every group the leaf counts is binned into spec->hist / spec->tail, nothing is written per group
@@ -125,7 +129,7 @@ uint64_t tier2_table_slots(uint64_t n_kmers);
 void launch_partition_tier2(const DeviceInfo& di, const PartitionPlan& p, int k, const unsigned long long* d_fill,
                             const void* d_recs, const void* d_spill, const uint32_t* d_failed_ids, kmer_count_pair* d_slots,
                             uint64_t n_slots, kmer_count_pair* d_pairs, uint64_t capacity, DevStatus* d_status, cudaStream_t st,
-                            void (*mark)(void*, const char*), void* mark_arg, const SpecOut* spec = nullptr);
+                            void (*mark)(void*, const char*), void* mark_arg, const SpecOut* spec = nullptr, bool canon = false);
 // sharded counting, owner side: the coarse partitions received from every source GPU ([src][n_coarse][coarse_cap] records,
 // [src][n_coarse] fills) are split into this GPU's fine buckets (p: n_buckets = n_coarse << fine_shift, cap, spill list)
 // Source s's segments for THIS owner are src.recs[s] ([n_coarse][coarse_cap] records) and src.fill[s] ([n_coarse] fills): plain

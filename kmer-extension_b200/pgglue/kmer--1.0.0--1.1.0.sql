@@ -22,6 +22,27 @@ CREATE FUNCTION kmer_gpu_count_spectrum(dna[], integer)
     AS 'MODULE_PATHNAME', 'kmer_gpu_count_spectrum'
     LANGUAGE C IMMUTABLE STRICT PARALLEL SAFE;
 
+-- Canonical k-mers: a k-mer and its reverse complement (a<->t, c<->g, order reversed) are one group, keyed by the smaller of
+-- the two texts -- the counting mode of `jellyfish count -C` and what GenomeScope expects of reads from both strands:
+--   SELECT * FROM kmer_gpu_canonical_counts(ARRAY(SELECT dna FROM reads), 21)
+--     ==  SELECT least(g.kmer::text COLLATE "C", reverse(translate(g.kmer::text, 'acgt', 'tgca')))::kmer AS kmer, count(*)
+--         FROM reads r, generate_kmers(r.dna, 21) AS g(kmer) GROUP BY 1
+CREATE FUNCTION kmer_gpu_canonical_counts(dna[], integer)
+    RETURNS TABLE (kmer kmer, count bigint)
+    AS 'MODULE_PATHNAME', 'kmer_gpu_canonical_counts'
+    LANGUAGE C IMMUTABLE STRICT PARALLEL SAFE;
+
+-- The abundance spectrum of that canonical GROUP BY:
+--   SELECT * FROM kmer_gpu_canonical_count_spectrum(ARRAY(SELECT dna FROM reads), 21)
+--     ==  SELECT cnt AS count, count(*) AS kmers
+--         FROM (SELECT count(*) AS cnt FROM reads r, generate_kmers(r.dna, 21) AS g(kmer)
+--               GROUP BY least(g.kmer::text COLLATE "C", reverse(translate(g.kmer::text, 'acgt', 'tgca')))) s
+--         GROUP BY cnt ORDER BY cnt
+CREATE FUNCTION kmer_gpu_canonical_count_spectrum(dna[], integer)
+    RETURNS TABLE (count bigint, kmers bigint)
+    AS 'MODULE_PATHNAME', 'kmer_gpu_canonical_count_spectrum'
+    LANGUAGE C IMMUTABLE STRICT PARALLEL SAFE;
+
 -- equals / starts_with / contains over a column of k-mers against one constant (kmer.c:226-285):
 --   element i of the result:  op 0  kmer[i] = $2      op 1  kmer[i] ^@ $2      op 2  $2::qkmer @> kmer[i]
 CREATE FUNCTION kmer_gpu_match(kmer[], text, integer)

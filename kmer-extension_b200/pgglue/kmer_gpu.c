@@ -12,6 +12,8 @@
  *                              calls (kmer.c:226-285).
  *   kmer_gpu_spectrum_datums(): the k-mer abundance spectrum (count of counts) of that GROUP BY, binned on the GPU:
  *                              (count, number of k-mers with that count) rows, ascending by count.
+ *   kmer_gpu_canonical_count_datums() / kmer_gpu_canonical_spectrum_datums(): the same for canonical k-mers (a k-mer and
+ *                              its reverse complement are one group, keyed by the smaller of the two).
  *
  * Results are palloc'ed in the caller's memory context, exactly like the reference's functions
  * (kmer.c:92,124,341); `kmer` results carry the 1-byte short varlena header generate_kmers writes
@@ -43,6 +45,11 @@
  *       --   ==  SELECT cnt AS count, count(*) AS kmers
  *       --       FROM (SELECT count(*) AS cnt FROM reads r, generate_kmers(r.dna, 21) AS g(kmer) GROUP BY g.kmer) s
  *       --       GROUP BY cnt ORDER BY cnt
+ *   CREATE FUNCTION kmer_gpu_canonical_counts(dna[], integer) RETURNS TABLE (kmer kmer, count bigint)
+ *       AS 'MODULE_PATHNAME', 'kmer_gpu_canonical_counts' LANGUAGE C IMMUTABLE STRICT PARALLEL SAFE;
+ *   CREATE FUNCTION kmer_gpu_canonical_count_spectrum(dna[], integer) RETURNS TABLE (count bigint, kmers bigint)
+ *       AS 'MODULE_PATHNAME', 'kmer_gpu_canonical_count_spectrum' LANGUAGE C IMMUTABLE STRICT PARALLEL SAFE;
+ *       -- the two above with the k-mer least(kmer::text COLLATE "C", reverse(translate(kmer::text, 'acgt', 'tgca')))::kmer
  */
 
 
@@ -93,9 +100,9 @@ kmer_gpu_context(void)
  * dnas[0..n) are detoasted `dna` datums (PG_DETOAST_DATUM in the caller).  On return *kmers is an array
  * of *n_groups `kmer` datums (short-header varlenas) and *counts their bigint counts.
  */
-void
-kmer_gpu_count_datums(struct varlena **dnas, uint64_t n, int k, struct varlena ***kmers, int64_t **counts,
-					  uint64_t *n_groups)
+static void
+count_datums(struct varlena **dnas, uint64_t n, int k, bool canonical, struct varlena ***kmers, int64_t **counts,
+			 uint64_t *n_groups)
 {
 	kmer_cuda_ctx *ctx = kmer_gpu_context();
 	uint64_t *off = (uint64_t *) palloc((n + 1) * sizeof(uint64_t));
@@ -117,7 +124,8 @@ kmer_gpu_count_datums(struct varlena **dnas, uint64_t n, int k, struct varlena *
 
 	/* split result format: groups with count 1 come back as bare codes, the rest as (code, count) pairs --
 	 * the same table as kmer_cuda_submit_count(), half the bytes across PCIe on mostly distinct k-mers */
-	if (kmer_cuda_submit_count_split(ctx, flat, off, n, k, &uniq, &n_uniq, &pairs, &n_pairs, &n_kmers) != KMER_OK)
+	if ((canonical ? kmer_cuda_submit_count_canonical(ctx, flat, off, n, k, &uniq, &n_uniq, &pairs, &n_pairs, &n_kmers)
+				   : kmer_cuda_submit_count_split(ctx, flat, off, n, k, &uniq, &n_uniq, &pairs, &n_pairs, &n_kmers)) != KMER_OK)
 		kmer_gpu_raise(kmer_cuda_last_error(ctx));
 	d = n_uniq + n_pairs;
 
@@ -169,6 +177,21 @@ kmer_gpu_count_datums(struct varlena **dnas, uint64_t n, int k, struct varlena *
 	*n_groups = d;
 }
 
+void
+kmer_gpu_count_datums(struct varlena **dnas, uint64_t n, int k, struct varlena ***kmers, int64_t **counts,
+					  uint64_t *n_groups)
+{
+	count_datums(dnas, n, k, false, kmers, counts, n_groups);
+}
+
+/* canonical k-mers: every group's k-mer is the smaller of a k-mer and its reverse complement */
+void
+kmer_gpu_canonical_count_datums(struct varlena **dnas, uint64_t n, int k, struct varlena ***kmers, int64_t **counts,
+								uint64_t *n_groups)
+{
+	count_datums(dnas, n, k, true, kmers, counts, n_groups);
+}
+
 /* counts below this are binned by the library; the (rare) groups above it come back whole and are folded in here */
 #define KMER_GPU_SPECTRUM_HIST_LEN 65536
 
@@ -184,8 +207,8 @@ cmp_u64(const void *a, const void *b)
  * dnas[0..n) as for kmer_gpu_count_datums.  On return (*counts)[i], (*kmers)[i] for i < *n_out are the rows of the spectrum:
  * every count that occurs, ascending, and the number of distinct k-mers with exactly that count.
  */
-void
-kmer_gpu_spectrum_datums(struct varlena **dnas, uint64_t n, int k, int64_t **counts, int64_t **kmers, uint64_t *n_out)
+static void
+spectrum_datums(struct varlena **dnas, uint64_t n, int k, bool canonical, int64_t **counts, int64_t **kmers, uint64_t *n_out)
 {
 	kmer_cuda_ctx *ctx = kmer_gpu_context();
 	uint64_t *off = (uint64_t *) palloc((n + 1) * sizeof(uint64_t));
@@ -203,7 +226,10 @@ kmer_gpu_spectrum_datums(struct varlena **dnas, uint64_t n, int k, int64_t **cou
 	flat = (char *) palloc(total + 16);
 	for (i = 0; i < n; i++)
 		memcpy(flat + off[i], VARDATA_ANY(dnas[i]), (size_t) (off[i + 1] - off[i]));
-	if (kmer_cuda_submit_count_spectrum(ctx, flat, off, n, k, KMER_GPU_SPECTRUM_HIST_LEN, &hist, &tail, &n_tail, &n_kmers) != KMER_OK)
+	if ((canonical ? kmer_cuda_submit_count_canonical_spectrum(ctx, flat, off, n, k, KMER_GPU_SPECTRUM_HIST_LEN, &hist, &tail,
+															   &n_tail, &n_kmers)
+				   : kmer_cuda_submit_count_spectrum(ctx, flat, off, n, k, KMER_GPU_SPECTRUM_HIST_LEN, &hist, &tail, &n_tail,
+													 &n_kmers)) != KMER_OK)
 		kmer_gpu_raise(kmer_cuda_last_error(ctx));
 
 	void *volatile r_hist = hist, *volatile r_tail = tail; /* pinned library buffers: released on every path */
@@ -248,6 +274,18 @@ kmer_gpu_spectrum_datums(struct varlena **dnas, uint64_t n, int k, int64_t **cou
 	kmer_cuda_release(ctx, r_hist);
 	kmer_cuda_release(ctx, r_tail);
 	*n_out = m;
+}
+
+void
+kmer_gpu_spectrum_datums(struct varlena **dnas, uint64_t n, int k, int64_t **counts, int64_t **kmers, uint64_t *n_out)
+{
+	spectrum_datums(dnas, n, k, false, counts, kmers, n_out);
+}
+
+void
+kmer_gpu_canonical_spectrum_datums(struct varlena **dnas, uint64_t n, int k, int64_t **counts, int64_t **kmers, uint64_t *n_out)
+{
+	spectrum_datums(dnas, n, k, true, counts, kmers, n_out);
 }
 
 /*
@@ -297,13 +335,12 @@ typedef struct CountsState
 	TupleDesc tupdesc;
 } CountsState;
 
-PG_FUNCTION_INFO_V1(kmer_gpu_counts);
 /*
  * kmer_gpu_counts(dna[], k) -> setof (kmer, bigint): value-per-call SRF like generate_kmers (kmer.c:289-351); the whole
- * batch is counted on the first call, in the multi-call memory context.
+ * batch is counted on the first call, in the multi-call memory context.  canonical: kmer_gpu_canonical_counts.
  */
-Datum
-kmer_gpu_counts(PG_FUNCTION_ARGS)
+static Datum
+counts_srf(FunctionCallInfo fcinfo, bool canonical)
 {
 	FuncCallContext *funcctx;
 	CountsState *st;
@@ -323,7 +360,8 @@ kmer_gpu_counts(PG_FUNCTION_ARGS)
 		funcctx = SRF_FIRSTCALL_INIT();
 		oldcontext = MemoryContextSwitchTo(funcctx->multi_call_memory_ctx);
 		if (get_call_result_type(fcinfo, NULL, &tupdesc) != TYPEFUNC_COMPOSITE)
-			ereport(ERROR, (errcode(ERRCODE_INTERNAL_ERROR), errmsg("kmer_gpu_counts must return a composite type")));
+			ereport(ERROR, (errcode(ERRCODE_INTERNAL_ERROR), errmsg("%s must return a composite type",
+																	canonical ? "kmer_gpu_canonical_counts" : "kmer_gpu_counts")));
 		deconstruct_array(arr, ARR_ELEMTYPE(arr), -1, false, 'i', &elems, &nulls, &n);
 		dnas = (struct varlena **) palloc((n ? n : 1) * sizeof(struct varlena *));
 		for (i = 0; i < n; i++)
@@ -331,7 +369,7 @@ kmer_gpu_counts(PG_FUNCTION_ARGS)
 				dnas[m++] = PG_DETOAST_DATUM(elems[i]);
 		st = (CountsState *) palloc(sizeof(CountsState));
 		st->tupdesc = BlessTupleDesc(tupdesc);
-		kmer_gpu_count_datums(dnas, (uint64_t) m, k, &st->kmers, &st->counts, &n_groups);
+		count_datums(dnas, (uint64_t) m, k, canonical, &st->kmers, &st->counts, &n_groups);
 		funcctx->max_calls = n_groups;
 		funcctx->user_fctx = st;
 		MemoryContextSwitchTo(oldcontext);
@@ -353,6 +391,21 @@ kmer_gpu_counts(PG_FUNCTION_ARGS)
 	SRF_RETURN_DONE(funcctx);
 }
 
+PG_FUNCTION_INFO_V1(kmer_gpu_counts);
+Datum
+kmer_gpu_counts(PG_FUNCTION_ARGS)
+{
+	return counts_srf(fcinfo, false);
+}
+
+PG_FUNCTION_INFO_V1(kmer_gpu_canonical_counts);
+/* kmer_gpu_canonical_counts(dna[], k) -> setof (kmer, bigint): one row per canonical k-mer, counted over both orientations */
+Datum
+kmer_gpu_canonical_counts(PG_FUNCTION_ARGS)
+{
+	return counts_srf(fcinfo, true);
+}
+
 typedef struct SpectrumState
 {
 	int64_t *counts;
@@ -360,13 +413,13 @@ typedef struct SpectrumState
 	TupleDesc tupdesc;
 } SpectrumState;
 
-PG_FUNCTION_INFO_V1(kmer_gpu_count_spectrum);
 /*
  * kmer_gpu_count_spectrum(dna[], k) -> setof (count bigint, kmers bigint), ascending by count: the abundance spectrum of
  * kmer_gpu_counts(dna[], k), computed without materialising the groups.  The batch is counted on the first call.
+ * canonical: kmer_gpu_canonical_count_spectrum, the spectrum of kmer_gpu_canonical_counts.
  */
-Datum
-kmer_gpu_count_spectrum(PG_FUNCTION_ARGS)
+static Datum
+spectrum_srf(FunctionCallInfo fcinfo, bool canonical)
 {
 	FuncCallContext *funcctx;
 	SpectrumState *st;
@@ -386,7 +439,9 @@ kmer_gpu_count_spectrum(PG_FUNCTION_ARGS)
 		funcctx = SRF_FIRSTCALL_INIT();
 		oldcontext = MemoryContextSwitchTo(funcctx->multi_call_memory_ctx);
 		if (get_call_result_type(fcinfo, NULL, &tupdesc) != TYPEFUNC_COMPOSITE)
-			ereport(ERROR, (errcode(ERRCODE_INTERNAL_ERROR), errmsg("kmer_gpu_count_spectrum must return a composite type")));
+			ereport(ERROR, (errcode(ERRCODE_INTERNAL_ERROR),
+							errmsg("%s must return a composite type",
+								   canonical ? "kmer_gpu_canonical_count_spectrum" : "kmer_gpu_count_spectrum")));
 		deconstruct_array(arr, ARR_ELEMTYPE(arr), -1, false, 'i', &elems, &nulls, &n);
 		dnas = (struct varlena **) palloc((n ? n : 1) * sizeof(struct varlena *));
 		for (i = 0; i < n; i++)
@@ -394,7 +449,7 @@ kmer_gpu_count_spectrum(PG_FUNCTION_ARGS)
 				dnas[m++] = PG_DETOAST_DATUM(elems[i]);
 		st = (SpectrumState *) palloc(sizeof(SpectrumState));
 		st->tupdesc = BlessTupleDesc(tupdesc);
-		kmer_gpu_spectrum_datums(dnas, (uint64_t) m, k, &st->counts, &st->kmers, &n_rows);
+		spectrum_datums(dnas, (uint64_t) m, k, canonical, &st->counts, &st->kmers, &n_rows);
 		funcctx->max_calls = n_rows;
 		funcctx->user_fctx = st;
 		MemoryContextSwitchTo(oldcontext);
@@ -413,6 +468,20 @@ kmer_gpu_count_spectrum(PG_FUNCTION_ARGS)
 		SRF_RETURN_NEXT(funcctx, tuple);
 	}
 	SRF_RETURN_DONE(funcctx);
+}
+
+PG_FUNCTION_INFO_V1(kmer_gpu_count_spectrum);
+Datum
+kmer_gpu_count_spectrum(PG_FUNCTION_ARGS)
+{
+	return spectrum_srf(fcinfo, false);
+}
+
+PG_FUNCTION_INFO_V1(kmer_gpu_canonical_count_spectrum);
+Datum
+kmer_gpu_canonical_count_spectrum(PG_FUNCTION_ARGS)
+{
+	return spectrum_srf(fcinfo, true);
 }
 
 PG_FUNCTION_INFO_V1(kmer_gpu_match);
